@@ -2,7 +2,7 @@
 """Benchmark of the WCT inference hot path (BASELINE.json metric: 512x512 five-level
 stylised frames/sec), one process per GPU.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference] [--dump-outputs DIR]
 
 A "step" = one pass of the hot path (WCT.predict semantics: encode style, then
 [encode -> WCT -> decode] x relu5_1..relu1_1, wct_tf semantics, alpha=0.8) over one batch
@@ -22,6 +22,11 @@ no work is shared or cached between frames).
 
 --impl reference: TensorFlow 1.x / Keras 2.0.9 are not installable offline, so the
 reference arm is the oracle port run on all host threads (kind "port").
+
+--dump-outputs DIR: after the timed steps, rank 0 writes the uint8 frames its last timed resident step
+returned as DIR/output.npy (float32, B x 512 x 512 x 3).  Inputs and weights are seeded, so two builds run
+with the same arguments can be compared output for output.  A batch above 64 MB in float32 is cut to a
+seeded sample of whole frames; DIR/output_frames.npy (float64) then lists which frames of the batch they are.
 """
 from __future__ import annotations
 
@@ -43,6 +48,7 @@ TARGETS = ["relu5_1", "relu4_1", "relu3_1", "relu2_1", "relu1_1"]
 SIZE = 512
 ALPHA = 0.8
 SEMANTICS = "tf"   # what stylize.py actually executes (model.py:154,158)
+DUMP_BYTES = 64 * 10 ** 6
 
 WORKLOAD = ("configs[1]: 5-level relu5_1->relu1_1, 512x512 content, 512x512 style per frame, alpha=0.8, "
             "wct_tf semantics")
@@ -160,21 +166,12 @@ def run_reference(args):
     torch.set_num_threads(threads)
     weights = make_synthetic_weights(42)
     c, s = frames(1, 1000), frames(1, 7)
-    budget = 240.0
-    t_used, times = 0.0, []
-    dt = 0.0
+    times = []
     for i in range(args.warmup + args.steps):
         t0 = time.time()
         nets.pipeline(c[0], s[0], weights, TARGETS, alpha=ALPHA, semantics=SEMANTICS, dtype=np.float32)
-        dt = time.time() - t0
-        t_used += dt
         if i >= args.warmup:
-            times.append(dt)
-        # bounded: stop early (>=1 timed step) rather than run past a few minutes
-        if times and t_used + dt > budget:
-            break
-    if not times:
-        times = [dt]
+            times.append(time.time() - t0)
     ms = 1000.0 * float(np.mean(times))
     value = 1000.0 / ms
     world = max(1, args.gpus)
@@ -193,6 +190,19 @@ def run_reference(args):
     }
     print(json.dumps(line))
     return 0
+
+
+def dump_outputs(d, frames_u8):
+    """Write the frames (uint8, B x H x W x 3) as float32 .npy files under d, at most DUMP_BYTES in all."""
+    os.makedirs(d, exist_ok=True)
+    frames_u8 = np.asarray(frames_u8)
+    per_frame = frames_u8[0].size * 4
+    fit = (DUMP_BYTES - 4096) // per_frame                         # 4 KB for the .npy headers and output_frames.npy
+    if frames_u8.shape[0] > fit:
+        idx = np.sort(np.random.default_rng(0).choice(frames_u8.shape[0], fit, replace=False))
+        np.save(os.path.join(d, "output_frames.npy"), idx.astype(np.float64))
+        frames_u8 = frames_u8[idx]
+    np.save(os.path.join(d, "output.npy"), frames_u8.astype(np.float32))
 
 
 def level_of_key(key):
@@ -220,8 +230,13 @@ def main():
     ap.add_argument("--no-fuse-pool", action="store_true", help="tuning: separate maxpool2 kernels after conv1_2/2_2/3_4/4_4")
     ap.add_argument("--no-roofline", action="store_true", help="skip the per-kernel profiling steps")
     ap.add_argument("--jacobi-tolq", type=float, default=0.0, help="tuning: eigensolver predicted-convergence level (0 = library default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the frames of the last timed step to DIR/output.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the frames of the GPU path; it does not apply to --impl reference")
         return run_reference(args)
 
     import torch
@@ -297,7 +312,7 @@ def main():
         n0 = eng.launches
         e0.record()
         for i in range(steps):
-            fn(i)
+            last = fn(i)
         e1.record()
         barrier()
         ms = e0.elapsed_time(e1)
@@ -306,14 +321,14 @@ def main():
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms, launches
+        return ms, launches, last
 
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    ms_total, launches = timed(step_resident, args.steps, args.warmup)
+    ms_total, launches, last_out = timed(step_resident, args.steps, args.warmup)
     clocks = sampler.stop() if rank == 0 else None
-    ms_e2e, _ = timed(step_e2e, args.steps, max(3, args.warmup // 2))
+    ms_e2e, _, _ = timed(step_e2e, args.steps, max(3, args.warmup // 2))
     eng.check_device()
 
     pk = peaks()
@@ -425,7 +440,7 @@ def main():
                                                 c_all, s_one)
             sharded_inputs = [(torch.from_numpy(frames(GB, 1000 + 1000 * j)).to(dev), torch.from_numpy(frames(1, 7 + 1000 * j)).to(dev))
                               for j in range(2)]
-            sharded_ms, _ = timed(sharded_step, max(3, args.steps // 2), 3)     # sharded compute + NCCL gather, event timed, max over ranks
+            sharded_ms, _, _ = timed(sharded_step, max(3, args.steps // 2), 3)     # sharded compute + NCCL gather, event timed, max over ranks
             sharded_ms /= max(3, args.steps // 2)
         else:
             for _ in range(3):
@@ -473,6 +488,8 @@ def main():
             "sharded_step_with_gather_ms": sharded_ms,
         }
         print(json.dumps(line))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last_out.cpu().numpy())
     if world > 1:
         dist.destroy_process_group()
     return 0

@@ -167,10 +167,13 @@ def test_frame_sharding_world2_gloo(B, tmp_path):
 
 def test_t7_reader_against_reference_torchfile(tmp_path):
     """A VGG .t7 written by tests/t7_writer.py is read identically by the reference's own
-    torchfile.py (vgg_normalised.py:16, force_8bytes_long=True) and by wct_tf_b200.t7."""
+    torchfile.py (vgg_normalised.py:16, force_8bytes_long=True) and by wct_tf_b200.t7.  What the
+    reference read from this very file is stored in tests/golden/reference_reads.npz
+    (tests/golden/make_reference_reads.py)."""
+    from tests.golden import make_reference_reads as R
     from tests.t7_writer import write_vgg_t7
     from wct_tf_b200 import t7, weights as W
-    w = W.make_synthetic_weights(5, relu_targets=["relu3_1"])
+    w = W.make_synthetic_weights(R.T7_SEED, relu_targets=R.T7_TARGETS)
     path = str(tmp_path / "vgg_normalised.t7")
     write_vgg_t7(path, w["vgg"])
     ours = t7.load_vgg_t7(path, deepest="relu5_1")
@@ -178,19 +181,13 @@ def test_t7_reader_against_reference_torchfile(tmp_path):
     for a, b in zip(ours, w["vgg"]):
         assert np.array_equal(a["weight"], b["weight"]) and np.array_equal(a["bias"], b["bias"])
     assert [l["name"] for l in t7.load_vgg_t7(path, deepest="relu2_1")][-1] == "conv2_1"    # stops at the target (vgg_normalised.py:48)
-    ref_path = "/root/reference/torchfile.py"
-    if os.path.exists(ref_path):
-        import importlib.util
-        spec = importlib.util.spec_from_file_location("_ref_torchfile", ref_path)
-        tf = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(tf)
-        net = tf.load(path, force_8bytes_long=True)
-        convs = [m for m in net.modules if m._typename == b"nn.SpatialConvolution"]
-        assert len(convs) == len(ours)
-        for m, o in zip(convs, ours):
-            assert np.array_equal(np.asarray(m.weight), o["weight"]) and np.array_equal(np.asarray(m.bias), o["bias"])
-        names = [m.name.decode() for m in net.modules[1:] if m._typename == b"nn.SpatialConvolution"]
-        assert names == [l["name"] for l in ours[1:]]
+    ref = np.load(os.path.join(ROOT, "tests", "golden", "reference_reads.npz"))
+    assert R.file_digest(path) == str(ref["torchfile_t7_sha256"]), "not the file the reference read (writer or weights drifted)"
+    convs = [str(d) for d in ref["torchfile_conv_digests"]]
+    assert len(convs) == len(ours)
+    for d, o in zip(convs, ours):
+        assert R.array_digest(o["weight"], o["bias"]) == d, o["name"]
+    assert [str(n) for n in ref["torchfile_conv_names"]] == [l["name"] for l in ours[1:]]
     # and through the public loader: checkpoints stay .npz
     ck = str(tmp_path / "dec.npz")
     W.save_weights(ck, w)

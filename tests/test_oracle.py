@@ -29,13 +29,16 @@ def test_wct_np_restatement_matches_reference_golden(path):
     assert ref_ops.spectral_gap_ok(g["wc"]) and ref_ops.spectral_gap_ok(g["ws"])
 
 
-def test_live_reference_import_if_present():
-    ref = ref_ops.load_reference_ops()
-    if ref is None:
-        pytest.skip("/root/reference not present (GPU box)")
-    g = np.load(GOLDEN[0])
-    out = ref.wct_np(g["content"], g["style"], float(g["alpha"]))
-    assert np.array_equal(out, g["out_ref_fp32"])
+REF_READS = os.path.join(os.path.dirname(__file__), "golden", "reference_reads.npz")
+
+
+def test_reference_wct_np_reproduces_fixture():
+    """The reference's own ops.wct_np, re-run on a fixture's inputs (tests/golden/make_reference_reads.py), returns the
+    fixture's out_ref_fp32 bit for bit."""
+    from tests.golden.make_reference_reads import array_digest
+    ref = np.load(REF_READS)
+    g = np.load(os.path.join(os.path.dirname(__file__), "golden", str(ref["wct_np_fixture"])))
+    assert array_digest(g["out_ref_fp32"]) == str(ref["wct_np_out_sha256"])
 
 
 def test_np_vs_tf_semantics_differ_only_as_documented():
@@ -130,22 +133,14 @@ def test_oracle_pipeline_matches_reference_code_fixture(path):
     assert np.abs(o32 - g["out_ref_fp32"]).max() <= max(1e-4, 4 * noise)
 
 
-def test_reference_code_live_reproduces_fixture_if_present(tmp_path):
-    if not os.path.exists("/root/reference/model.py"):
-        pytest.skip("reference tree not mounted")
-    from tests.golden import np_tf1
-    from tests.t7_writer import write_vgg_t7
-    path = [p for p in PIPE_GOLDEN if "wct_31_11_odd" in p][0]
-    g, targets, w = load_pipeline_fixture(path)
-    t7 = str(tmp_path / "vgg.t7")
-    write_vgg_t7(t7, w["vgg"])
-    dec = {l["name"]: (l["kernel"], l["bias"]) for t in targets for l in w["decoders"][t]}
-    with np_tf1.reference_modules() as ref:
-        out, levels = np_tf1.run_reference(ref, g["content"][None] / 255.0, g["style"][None] / 255.0, t7, dec, targets,
-                                           float(g["alpha"]), bool(g["adain"]), np.float64, swap5=bool(g["swap5"]),
-                                           ss_alpha=float(g["ss_alpha"]))
+def test_reference_code_reproduces_pipeline_fixture():
+    """The reference's WCTModel code (over tests/golden/np_tf1.py), re-run in float64 on a fixture's inputs and weights
+    (tests/golden/make_reference_reads.py), returns the fixture's out_ref_fp64."""
+    ref = np.load(REF_READS)
+    g, _, _ = load_pipeline_fixture(os.path.join(os.path.dirname(__file__), "golden", str(ref["pipeline_fixture"])))
+    out = ref["pipeline_out_fp64"]
+    assert out.shape == g["out_ref_fp64"].shape
     assert np.abs(out - g["out_ref_fp64"]).max() <= 1e-12
-    assert "tensorflow" not in __import__("sys").modules or not hasattr(__import__("sys").modules["tensorflow"], "placeholder_with_default")
 
 
 # ---------------------------------------------------------------------------
