@@ -178,6 +178,28 @@ WCTB200_API int wctb200_adain_level(const void* content, int Nc, int Hc, int Wc,
                         const void* style, int Ns, int Hs, int Ws, int C,
                         float alpha, float eps, void* out, void* ws, size_t ws_bytes, void* stream);
 
+/* ---- spatial control: one style per region of a label mask (Li et al. 2017, sec. 4) ---------------------------------- *
+ * A uint8 label map [Nc][Hc][Wc] at the resolution of the features splits every content frame into regions.  Label r < R
+ * selects style r: the frame's features RESTRICTED to the pixels labelled r are transformed with their own statistics
+ * (means, covariance, k_c, alpha blend and mean re-add of wct_tf / wct_np / adain) and the result is written back to those
+ * pixels.  Labels >= R ("keep"), and every region with fewer than 2 pixels, leave the output equal by value to the input.
+ * R in 1..8; the R styles are shared by all frames. */
+/* nearest-neighbour resize of uint8 label maps in exact integer arithmetic:
+ * dst[n][y][x] = src[n][(y*Hs) div Hd][(x*Ws) div Wd]; src [N][Hs][Ws], dst [N][Hd][Wd] (device) */
+WCTB200_API int wctb200_labels_resize_nearest(const uint8_t* src, int N, int Hs, int Ws, int Hd, int Wd, uint8_t* dst, void* stream);
+/* device scratch for wctb200_wct_apply_regions and wctb200_adain_regions */
+WCTB200_API size_t wctb200_wct_regions_workspace_bytes(int C, int Nc, int R);
+/* labels: device uint8 [Nc][Hc][Wc] at feature resolution; states: HOST array of R device pointers, each a
+   wctb200_wct_style_state of Ns = 1.  k_out (may be NULL): int32 [2*Nc*R] = k_c per (frame, region), frame-major,
+   then the pixel count n_r of each. */
+WCTB200_API int wctb200_wct_apply_regions(const void* content, int Nc, int Hc, int Wc, int C, const uint8_t* labels, int R,
+                              const void* const* states, float alpha, float eps_cov, float eps_eig, float thresh,
+                              int readd_content_mean, void* out, int32_t* k_out, void* ws, size_t ws_bytes, void* stream);
+/* styles: HOST array of R device pointers to SPF16 [1,Hs_r,Ws_r,C]; style_hw: HOST int [R][2] */
+WCTB200_API int wctb200_adain_regions(const void* content, int Nc, int Hc, int Wc, int C, const uint8_t* labels, int R,
+                          const void* const* styles, const int* style_hw, float alpha, float eps,
+                          void* out, void* ws, size_t ws_bytes, void* stream);
+
 /*
  * wct_style_swap (ops.py:145-217) + style_swap (ops.py:219-278) for ONE content/style pair: whiten both encodings, take every
  * patch x patch window of the whitened style at `stride` (--ss-patch-size / --ss-stride, stylize.py:33-34), replace every

@@ -6,6 +6,9 @@ content x style loop at stylize.py:70-119, output naming ``<content>_<style><ext
   python stylize.py --checkpoints DIR5 DIR4 ... --relu-targets relu5_1 relu4_1 ... --vgg-path vgg_normalised.t7 \
       --content-path IN --style-path STYLE --out-path OUT --alpha 0.8
 
+Spatial control: ``--mask-path MASK --mask-styles S0 S1 ...`` stylises the pixels labelled r in the 8-bit mask (mode L or P)
+with style Sr and leaves labels >= the number of styles unstyled; the output is ``<content>_<mask stem><ext>``.
+
 ``--checkpoints`` are TF1 checkpoint directories or ``.npz`` bundles, ``--vgg-path`` a Torch7 ``.t7`` or ``.npz`` file
 (wct_tf_b200.weights.load_weights); ``--synthetic-weights SEED`` runs with seeded random weights when the published
 models are not on disk (offline build).
@@ -43,6 +46,8 @@ _FLAGS = [
     # not in the reference
     (("--synthetic-weights",), dict(type=int, default=None, help="seeded random weights (no model files needed)")),
     (("--semantics",), dict(type=str, default="tf", choices=["tf", "np"], help="wct_tf (the reference graph) or wct_np eps/blend rules")),
+    (("--mask-path",), dict(type=str, default=None, help="8-bit label mask (mode L or P): label r takes --mask-styles[r], others keep the content")),
+    (("--mask-styles",), dict(nargs="+", type=str, default=None, help="one style image per mask label 0, 1, ... (at most 8)")),
 ]
 
 
@@ -51,6 +56,21 @@ def build_parser():
     for names, kw in _FLAGS:
         parser.add_argument(*names, **kw)
     return parser
+
+
+def parse_args(argv=None):
+    """Parse and check the flag combinations the mask mode does not support."""
+    parser = build_parser()
+    args = parser.parse_args(argv)
+    if args.mask_path is not None or args.mask_styles is not None:
+        if args.mask_path is None or not args.mask_styles:
+            parser.error("--mask-path and --mask-styles go together")
+        if len(args.mask_styles) > 8:
+            parser.error("--mask-styles takes at most 8 styles")
+        for flag, on in (("--swap5", args.swap5), ("--concat", args.concat), ("-r/--random", args.random > 0)):
+            if on:
+                parser.error("%s cannot be combined with --mask-path" % flag)
+    return args
 
 
 def _listing(path, io):
@@ -67,6 +87,24 @@ def _prepare_style(path, args, io, dimg, content_dev, device):
     if args.keep_colors:
         img = dimg.preserve_colors_np(img, content_dev)
     return img
+
+
+def _stylize_masked(model, content_dev, styles_dev, labels_dev, args):
+    """The --mask-path form of _stylize_pair: the labels ride along every pass."""
+    kw = dict(alpha=args.alpha, adain=args.adain, return_device=True, passes=args.passes, labels=labels_dev)
+    return model.predict_batch(content_dev, list(styles_dev), **kw)[0]
+
+
+def _load_mask(path, content_dev, device):
+    """The mask as cuda uint8 [1, H, W] at the content's size (nearest-neighbour resize on the device when it differs)."""
+    import torch
+    from wct_tf_b200 import imageio as io
+    mask = torch.from_numpy(io.get_mask(path)).to(device).unsqueeze(0)
+    H, W = content_dev.shape[-3], content_dev.shape[-2]
+    if tuple(mask.shape[1:]) != (H, W):
+        from wct_tf_b200 import device_image as dimg
+        mask = dimg.labels_resize(mask, H, W)
+    return mask
 
 
 def _stylize_pair(model, content_dev, style_dev, args):
@@ -91,13 +129,13 @@ def make_model(args):
 
 
 def main(argv=None):
-    args = build_parser().parse_args(argv)
+    args = parse_args(argv)
     from wct_tf_b200 import device_image as dimg
     from wct_tf_b200 import imageio as io
     t_start = time.time()
     model = make_model(args)
-    styles = _listing(args.style_path, io)
-    if os.path.isdir(args.style_path) and args.random > 0:
+    styles = _listing(args.style_path, io) if args.mask_path is None else []
+    if args.mask_path is None and os.path.isdir(args.style_path) and args.random > 0:
         styles = list(np.random.choice(styles, args.random))
     os.makedirs(args.out_path, exist_ok=True)
 
@@ -108,6 +146,15 @@ def main(argv=None):
         content_dev = dimg.to_device(io.get_img(content_path), device)
         if args.content_size > 0:
             content_dev = dimg.resize_to(content_dev, args.content_size)
+        if args.mask_path is not None:
+            labels = _load_mask(args.mask_path, content_dev, device)
+            region_styles = [_prepare_style(p, args, io, dimg, content_dev, device) for p in args.mask_styles]
+            result = _stylize_masked(model, content_dev, region_styles, labels, args)
+            target = os.path.join(args.out_path, "{}_{}{}".format(stem, os.path.splitext(os.path.basename(args.mask_path))[0], ext))
+            io.save_img(target, result.cpu().numpy())
+            written += 1
+            print("{}: Wrote stylized output image to {}".format(written, target))
+            continue
         for style_path in styles:
             style_dev = _prepare_style(style_path, args, io, dimg, content_dev, device)
             result = _stylize_pair(model, content_dev, style_dev, args)

@@ -51,6 +51,10 @@ SIGNATURES = {
     "wctb200_jacobi_eigh": (_i, [_vp, _i, _i, _vp, _vp, _vp]),
     "wctb200_style_swap_workspace_bytes": (_sz, [_i, _i, _i, _i, _i, _i, _i]),
     "wctb200_style_swap_level": (_i, [_vp, _i, _i, _vp, _i, _i, _i, _i, _i, _f, _f, _f, _vp, _vp, _vp, _sz, _vp]),
+    "wctb200_labels_resize_nearest": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp]),
+    "wctb200_wct_regions_workspace_bytes": (_sz, [_i, _i, _i]),
+    "wctb200_wct_apply_regions": (_i, [_vp, _i, _i, _i, _i, _vp, _i, _vp, _f, _f, _f, _f, _i, _vp, _vp, _vp, _sz, _vp]),
+    "wctb200_adain_regions": (_i, [_vp, _i, _i, _i, _i, _vp, _i, _vp, _vp, _f, _f, _vp, _vp, _sz, _vp]),
 }
 
 # tuning / probe hooks (wct_tf_b200/csrc/wctb200_debug.h): NOT part of the ABI, bound for tools/ and tests/ only

@@ -110,6 +110,14 @@ int launch_wct_style_prepare(const __half*, int, int, int, int, float, float, fl
 int launch_wct_apply(const __half*, int, int, int, int, const void*, int, float, float, float, float, int, __half*, int32_t*,
                      void*, size_t, cudaStream_t);
 int launch_covariance(const __half*, int, int, int, int, float, float*, float*, cudaStream_t);
+int launch_labels_nearest(const uint8_t* src, int N, int Hs, int Ws, int Hd, int Wd, uint8_t* dst, cudaStream_t st);
+size_t wct_regions_workspace_bytes(int C, int Nc, int R);
+int launch_wct_apply_regions(const __half* content, int Nc, int Hc, int Wc, int C, const uint8_t* labels, int R,
+                             const void* const* states, float alpha, float eps_cov, float eps_eig, float thresh, int readd,
+                             __half* out, int32_t* k_out, void* ws, size_t ws_bytes, cudaStream_t st);
+int launch_adain_regions(const __half* content, int Nc, int Hc, int Wc, int C, const uint8_t* labels, int R,
+                         const __half* const* styles, const int* style_hw, float alpha, float eps, __half* out, void* ws,
+                         size_t ws_bytes, cudaStream_t st);
 int launch_jacobi(float*, int, int, float*, int*, cudaStream_t, const int* skip);
 int launch_eig_post(const float*, const float*, float*, int, int, float, float, int, float*, float*, int*, cudaStream_t, const int* skip);
 extern int g_conv_bn_override;
@@ -304,6 +312,38 @@ int wctb200_adain_level(const void* content, int Nc, int Hc, int Wc, const void*
     WCTB_REQUIRE(geom_ok(Nc, Hc, Wc, C) && geom_ok(Ns, Hs, Ws, C), "adain_level: bad geometry");
     return launch_adain_level(HCP(content), Nc, Hc, Wc, HCP(style), Ns, Hs, Ws, C, alpha, eps, HP(out), ws, ws_bytes,
                               ST(stream));
+}
+
+int wctb200_labels_resize_nearest(const uint8_t* src, int N, int Hs, int Ws, int Hd, int Wd, uint8_t* dst, void* stream) {
+    WCTB_REQUIRE(src && dst, "labels_resize_nearest: null pointer");
+    WCTB_REQUIRE(N >= 1 && Hs >= 1 && Ws >= 1 && Hd >= 1 && Wd >= 1 && Hs <= (1 << 15) && Ws <= (1 << 15) && Hd <= (1 << 15) &&
+                     Wd <= (1 << 15) && (long long)N * Hd * Wd < (1ll << 40),
+                 "labels_resize_nearest: bad geometry N=%d %dx%d -> %dx%d", N, Hs, Ws, Hd, Wd);
+    return launch_labels_nearest(src, N, Hs, Ws, Hd, Wd, dst, ST(stream));
+}
+size_t wctb200_wct_regions_workspace_bytes(int C, int Nc, int R) {
+    if (C < 8 || Nc < 1 || R < 1 || R > 8) return 0;
+    return wct_regions_workspace_bytes(C, Nc, R);
+}
+int wctb200_wct_apply_regions(const void* content, int Nc, int Hc, int Wc, int C, const uint8_t* labels, int R,
+                              const void* const* states, float alpha, float eps_cov, float eps_eig, float thresh,
+                              int readd_content_mean, void* out, int32_t* k_out, void* ws, size_t ws_bytes, void* stream) {
+    WCTB_REQUIRE(content && labels && states && out && ws, "wct_apply_regions: null pointer");
+    WCTB_REQUIRE(R >= 1 && R <= 8, "wct_apply_regions: R=%d not in 1..8", R);
+    WCTB_REQUIRE(geom_ok(Nc, Hc, Wc, C), "wct_apply_regions: bad geometry");
+    return launch_wct_apply_regions(HCP(content), Nc, Hc, Wc, C, labels, R, states, alpha, eps_cov, eps_eig, thresh,
+                                    readd_content_mean, HP(out), k_out, ws, ws_bytes, ST(stream));
+}
+int wctb200_adain_regions(const void* content, int Nc, int Hc, int Wc, int C, const uint8_t* labels, int R,
+                          const void* const* styles, const int* style_hw, float alpha, float eps, void* out, void* ws,
+                          size_t ws_bytes, void* stream) {
+    WCTB_REQUIRE(content && labels && styles && style_hw && out && ws, "adain_regions: null pointer");
+    WCTB_REQUIRE(R >= 1 && R <= 8, "adain_regions: R=%d not in 1..8", R);
+    WCTB_REQUIRE(geom_ok(Nc, Hc, Wc, C), "adain_regions: bad geometry");
+    for (int r = 0; r < R; ++r)
+        WCTB_REQUIRE(geom_ok(1, style_hw[2 * r], style_hw[2 * r + 1], C), "adain_regions: bad geometry of style %d", r);
+    return launch_adain_regions(HCP(content), Nc, Hc, Wc, C, labels, R, reinterpret_cast<const __half* const*>(styles), style_hw,
+                                alpha, eps, HP(out), ws, ws_bytes, ST(stream));
 }
 
 int wctb200_covariance(const void* act, int N, int H, int W, int C, float eps_cov, float* mean, float* cov, void* stream) {

@@ -423,7 +423,8 @@ int scratch_alloc(void** ptr, size_t bytes, cudaStream_t st, int slot);
 // ---------------------------------------------------------------------------
 enum ConvMode { CONV_3X3 = 0, CONV_APPLY = 1, CONV_UP2 = 2, CONV_TAPS = 3 };
 int launch_conv_tc(int mode, const __half* in, int N, int H, int W, int Cin, const __half* w_split, int nsets,
-                   const float* wscale, const float* bias, int Cout, int flags, __half* out, cudaStream_t st, int kw = 3);
+                   const float* wscale, const float* bias, int Cout, int flags, __half* out, cudaStream_t st, int kw = 3,
+                   const uint8_t* labels = nullptr, int R = 1, const uint32_t* tilemask = nullptr);
 // trailer of a prepared weight buffer: [0] = 1/scale (float), see wctb200_prep_conv_weights
 static inline const float* weight_scale_ptr(const __half* w_split, int taps_total, int Cin, int Cout) {
     return reinterpret_cast<const float*>(w_split + (size_t)2 * taps_total * Cin * Cout);

@@ -60,6 +60,11 @@ struct ConvParams {
     const float* wscale;  // device scalar: 1 / (power-of-two scale the weights were stored with), or nullptr (= 1)
     __half* out;          // SPF16, Cout channels; UP2: [N, 2H, 2W, Cout]
     unsigned int* err;
+    // APPLY per region (wctb200_wct_apply_regions): work items are (tile, region) pairs, weight / bias set image*R + region;
+    // tilemask[image][tile] bit r = the tile holds a pixel of region r that is transformed, the epilogue stores only those
+    const uint8_t* labels;      // [N][H][W] or nullptr
+    const uint32_t* tilemask;   // [N][tiles_per_image]
+    int R;
 };
 
 // ===========================================================================
@@ -108,8 +113,11 @@ struct TileCoord {
     long long p0, p_end;
     int n0, set;
     int cls;              // UP2: output parity class a*2+b
+    int region;           // APPLY per region: the region this work item stores
+    bool skip;            // APPLY per region: the tile holds no pixel of the region (every role skips the item)
 };
 
+template <bool REG>
 __device__ __forceinline__ TileCoord tile_coord(const ConvParams& p, int tile, int n_tiles, int BN) {
     TileCoord t;
     const int nt = tile % n_tiles;
@@ -117,7 +125,19 @@ __device__ __forceinline__ TileCoord tile_coord(const ConvParams& p, int tile, i
     const long long HpWp = (long long)p.Hp * p.Wp;
     t.n0 = nt * BN;
     t.cls = 0;
-    if (p.pool) {
+    t.region = 0;
+    t.skip = false;
+    if (REG) {
+        // region fastest after the cout tile: the R items of one position tile run together and share its A tiles in L2
+        t.region = mt % p.R;
+        mt /= p.R;
+        const int img = mt / p.tiles_per_image;
+        const int r = mt - img * p.tiles_per_image;
+        t.p0 = img * HpWp + (long long)r * 128;
+        t.p_end = (img + 1) * HpWp;
+        t.set = img * p.R + t.region;
+        t.skip = ((__ldg(p.tilemask + mt) >> t.region) & 1u) == 0u;
+    } else if (p.pool) {
         // mt = (image * row pairs + pair i) * column segments + t; rows 2i, 2i+1, interior columns [64t, 64t + 64)
         const int t_ = mt % p.pool_tx;
         const int r_ = mt / p.pool_tx;
@@ -148,7 +168,8 @@ __device__ __forceinline__ TileCoord tile_coord(const ConvParams& p, int tile, i
     return t;
 }
 
-template <int BN, bool FUSE_>
+// REG: the per-region apply (ConvParams::labels); a template parameter so that every other conv compiles as before
+template <int BN, bool FUSE_, bool REG>
 __global__ void __launch_bounds__(Conv2Cfg<BN, FUSE_>::THREADS, 1)
 conv_tc2_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
                 const __grid_constant__ CUtensorMap mapA64, const ConvParams p, const int total_tiles, const int n_tiles) {
@@ -200,7 +221,8 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant_
         if (lane == 0) {
             uint32_t itg = 0;
             for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
-                const TileCoord tc = tile_coord(p, tile, n_tiles, BN);
+                const TileCoord tc = tile_coord<REG>(p, tile, n_tiles, BN);
+                if (REG && tc.skip) continue;        // the MMA and epilogue warps skip the same items (same tile_coord)
                 for (int it = 0; it < kiters; ++it, ++itg) {
                     const int s = itg % Cfg::STAGES;
                     const uint32_t ph = (itg / Cfg::STAGES) & 1;
@@ -237,6 +259,7 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant_
             constexpr uint32_t idesc2 = umma_idesc_f16(Cfg::BM, Cfg::FUSE ? 2 * BN : BN);
             uint32_t itg = 0, cg_ = 0;
             for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
+                if (REG && tile_coord<REG>(p, tile, n_tiles, BN).skip) continue;
                 for (int c = 0; c < nchunks; ++c, ++cg_) {
                     const int b = cg_ % Cfg::NBUF;
                     const uint32_t bph = (cg_ / Cfg::NBUF) & 1;
@@ -289,7 +312,8 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant_
         const float wsc = p.wscale ? __ldg(p.wscale) : 1.f;
         uint32_t cg_ = 0;
         for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
-            const TileCoord tc = tile_coord(p, tile, n_tiles, BN);
+            const TileCoord tc = tile_coord<REG>(p, tile, n_tiles, BN);
+            if (REG && tc.skip) continue;
             // stage this tile's bias slice (named barrier 1: epilogue warps only)
             asm volatile("bar.sync 1, %0;" ::"r"(ETHREADS) : "memory");
             for (int i = et; i < BN; i += ETHREADS) sbias[i] = p.bias ? p.bias[(long long)(p.mode == CONV_APPLY ? tc.set : 0) * p.Cout + tc.n0 + i] : 0.f;   // UP2: set = weight parity class, ONE bias
@@ -417,7 +441,8 @@ conv_tc2_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant_
                 const unsigned int r = pos - n * hpwp;
                 const int yy = (int)(r / (unsigned int)p.Wp);
                 const int xx = (int)(r - (unsigned int)yy * (unsigned int)p.Wp);
-                if (yy >= 1 && yy <= p.H && xx >= 1 && xx <= p.W && !*abort_flag) {
+                if (yy >= 1 && yy <= p.H && xx >= 1 && xx <= p.W && !*abort_flag &&
+                    (!REG || p.labels[((long long)n * p.H + (yy - 1)) * p.W + (xx - 1)] == tc.region)) {
                     int y = yy - 1, x = xx - 1;
                     if (up2) { y = 2 * y + (tc.cls >> 1); x = 2 * x + (tc.cls & 1); }
                     flags = halo_flags(go, y, x);
@@ -493,18 +518,18 @@ int make_tensor_map_3d(CUtensorMap* m, const void* base, uint64_t d0, uint64_t d
 
 int g_conv_oversub = 4;
 
-template <int BN, bool FUSE_>
+template <int BN, bool FUSE_, bool REG = false>
 static int launch2_bn(const CUtensorMap& mA, const CUtensorMap& mB, const CUtensorMap& mA64, const ConvParams& p, int total_tiles,
                       int n_tiles, cudaStream_t st) {
     using Cfg = Conv2Cfg<BN, FUSE_>;
-    WCTB_ENSURE_SMEM((conv_tc2_kernel<BN, FUSE_>), Cfg::SMEM_BYTES);
+    WCTB_ENSURE_SMEM((conv_tc2_kernel<BN, FUSE_, REG>), Cfg::SMEM_BYTES);
     // Over-subscribed persistent grid: with g_conv_oversub x #SMs CTAs (1 resident per SM) the
     // hardware block scheduler hands queued CTAs to whichever SMs are free, so a conv launched
     // while the Jacobi clusters of the other stream hold half the SMs still balances its tiles
     // (a grid of exactly #SMs would run as two unbalanced waves).
     int grid = device_sm_count() * (g_conv_oversub > 0 ? g_conv_oversub : 1);
     if (grid > total_tiles) grid = total_tiles;
-    conv_tc2_kernel<BN, FUSE_><<<grid, Cfg::THREADS, Cfg::SMEM_BYTES, st>>>(mA, mB, mA64, p, total_tiles, n_tiles);
+    conv_tc2_kernel<BN, FUSE_, REG><<<grid, Cfg::THREADS, Cfg::SMEM_BYTES, st>>>(mA, mB, mA64, p, total_tiles, n_tiles);
     WCTB_CHECK_LAUNCH("conv_tc2_kernel");
     return 0;
 }
@@ -517,13 +542,18 @@ int g_conv_bn_override = 0;  // test/tuning hook: force the N tile (64/128/256)
 // mode CONV_APPLY: in [N,H,W,Cin], w_split [nsets][2][Cout][Cin],     out [N,H,W,Cout]   (per-image weight sets)
 // mode CONV_UP2  : in [N,H,W,Cin] (edge halo), w_split [4][2][Cout][4*Cin], out [N,2H,2W,Cout]
 // mode CONV_TAPS : in [N,H,W,Cin], w_split [2][Cout][kw*kw*Cin],      out [N,H,W,Cout]: top-left anchored kw x kw correlation
+// APPLY with labels: nsets = N*R weight sets (image-major), work items (tile, region) skipped where tilemask says so
 int launch_conv_tc(int mode, const __half* in, int N, int H, int W, int Cin, const __half* w_split, int nsets,
-                   const float* wscale, const float* bias, int Cout, int flags, __half* out, cudaStream_t st, int kw) {
+                   const float* wscale, const float* bias, int Cout, int flags, __half* out, cudaStream_t st, int kw,
+                   const uint8_t* labels, int R, const uint32_t* tilemask) {
     WCTB_REQUIRE(N >= 1 && H >= 2 && W >= 2, "conv: bad geometry N=%d H=%d W=%d", N, H, W);
     WCTB_REQUIRE(Cin % 64 == 0 && Cout % 64 == 0 && Cin >= 64 && Cout >= 64, "conv: Cin=%d Cout=%d must be multiples of 64", Cin, Cout);
     WCTB_REQUIRE(mode == CONV_3X3 || mode == CONV_APPLY || mode == CONV_UP2 || mode == CONV_TAPS, "conv: bad mode %d", mode);
     WCTB_REQUIRE(mode != CONV_TAPS || (kw >= 1 && kw <= 16), "conv: bad filter width %d", kw);
-    WCTB_REQUIRE(nsets == 1 || (mode == CONV_APPLY && nsets == N), "conv: nsets must be 1 (or N in apply mode)");
+    if (!labels) R = 1;
+    WCTB_REQUIRE(!labels || (mode == CONV_APPLY && tilemask && R >= 1 && R <= 32 && nsets == N * R && !(flags & WCTB200_POOL2)),
+                 "conv: per-region apply needs the apply mode, a tile mask and N*R weight sets");
+    WCTB_REQUIRE(labels || nsets == 1 || (mode == CONV_APPLY && nsets == N), "conv: nsets must be 1 (or N in apply mode)");
     ActGeom gi(N, H, W, Cin);
     WCTB_REQUIRE(gi.P < (1ll << 31) - 4096, "conv: too many padded positions (%lld)", gi.P);
     WCTB_REQUIRE(mode != CONV_UP2 || ActGeom(N, 2 * H, 2 * W, Cout).P < (1ll << 31), "conv: too many output positions");
@@ -534,7 +564,7 @@ int launch_conv_tc(int mode, const __half* in, int N, int H, int W, int Cin, con
     WCTB_REQUIRE(!pool || (mode == CONV_3X3 && (H + 1) / 2 >= 2 && (W + 1) / 2 >= 2), "conv: POOL2 needs the 3x3 mode and a pooled output >= 2x2");
     int BN = Cout % 128 == 0 ? 128 : 64;   // 256-wide tiles leave only 2 pipeline stages: measured slower
     if (g_conv_bn_override && Cout % g_conv_bn_override == 0) BN = g_conv_bn_override;
-    if (pool && BN > 128) BN = 128;        // the pooling epilogue works on the 4-warp layouts
+    if ((pool || labels) && BN > 128) BN = 128;   // the pooling / per-region epilogues work on the 4-warp layouts
 
     CUtensorMap mA, mB;
     int rc = make_tensor_map_3d(&mA, in, (uint64_t)Cin, (uint64_t)gi.P, 2, (uint64_t)Cin * 2, (uint64_t)gi.plane * 2, 128);
@@ -555,7 +585,10 @@ int launch_conv_tc(int mode, const __half* in, int N, int H, int W, int Cin, con
     p.kw = kw;
     p.products = (mode == CONV_3X3 || mode == CONV_UP2) ? g_conv_products : 3;    // the knob only touches the encoder / decoder convs
     p.nsets = nsets;
-    p.per_image = nsets > 1 ? 1 : 0;
+    p.per_image = (nsets > 1 || labels) ? 1 : 0;
+    p.labels = labels;
+    p.tilemask = tilemask;
+    p.R = R;
     p.tiles_per_image = cdiv((long long)gi.Hp * gi.Wp, 128);
     p.pool = pool ? 1 : 0;
     p.pool_tx = cdiv(W, 64);
@@ -565,9 +598,16 @@ int launch_conv_tc(int mode, const __half* in, int N, int H, int W, int Cin, con
     p.wscale = wscale;
     p.out = out;
     p.err = device_error_word();
-    const int m_tiles = pool ? N * p.pool_ho * p.pool_tx : (p.per_image ? N * p.tiles_per_image : cdiv(gi.P, 128));
+    const int m_tiles = pool ? N * p.pool_ho * p.pool_tx : (p.per_image ? N * p.tiles_per_image * R : cdiv(gi.P, 128));
     const int n_tiles = Cout / BN;
     const int total = m_tiles * n_tiles * (mode == CONV_UP2 ? 4 : 1);
+    if (labels) {   // per-region apply: the same tile / fusion choice as the plain apply, so one region computes bit-identically
+        if (BN == 64) return g_conv_fuse == 0 ? launch2_bn<64, false, true>(mA, mB, mA64, p, total, n_tiles, st)
+                                              : launch2_bn<64, true, true>(mA, mB, mA64, p, total, n_tiles, st);
+        return (g_conv_fuse == 1 || (g_conv_fuse < 0 && (long long)taps * Cin >= 9 * 256))
+                   ? launch2_bn<128, true, true>(mA, mB, mA64, p, total, n_tiles, st)
+                   : launch2_bn<128, false, true>(mA, mB, mA64, p, total, n_tiles, st);
+    }
     switch (BN) {
         // fused [b_hi|b_lo] MMAs (Conv2Cfg::FUSE): always at BN=64 (4 TMEM buffers stay); at BN=128 the ring shrinks to 2
         // buffers, which only pays for long K loops (measured: Cin=128 -9 %, Cin>=256 +3..5 %)

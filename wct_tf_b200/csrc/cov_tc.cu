@@ -40,6 +40,10 @@ struct CovParams {
     float* part;                 // [N][nslots][C][C] fp32 partial products (upper block triangle)
     float* psum;                 // [N][ksplit][C] fp32 partial sums of (x - shift)
     unsigned int* err;
+    // per-region statistics (wctb200_wct_apply_regions): item i = frame * R + region reads frame i / R; pixels whose label
+    // [frame][y][x] is not the item's region are zeroed in the centring step like TMA's out-of-range pixels
+    const uint8_t* labels;       // [N][H][W] or nullptr
+    int R;                       // regions per frame (1 without labels)
 };
 
 struct CovCfg {
@@ -64,6 +68,8 @@ __device__ __forceinline__ void tma_load_5d_cov(void* smem_dst, const void* map,
         : "memory");
 }
 
+// REG: statistics per (frame, region) item (CovParams::labels); a template parameter so that the plain covariance compiles as before
+template <bool REG>
 __global__ void __launch_bounds__(CovCfg::THREADS, 1)
 cov_tc_kernel(const __grid_constant__ CUtensorMap mapX, const CovParams p) {
     using Cfg = CovCfg;
@@ -88,7 +94,9 @@ cov_tc_kernel(const __grid_constant__ CUtensorMap mapX, const CovParams p) {
     while (rem >= p.nb - bi) { rem -= p.nb - bi; ++bi; }
     const int bj = bi + rem;
     const bool diag = (bi == bj);
-    const int img = blockIdx.y;
+    const int img = blockIdx.y;                  // item: output slots
+    const int frame = REG ? img / p.R : img;     // image the tiles are read from
+    const int region = REG ? img - frame * p.R : 0;
     const int tiles_img = p.tiles_x * p.tiles_y;
     const int t0 = split * p.tiles_per_split;
     const int t1 = min(t0 + p.tiles_per_split, tiles_img);
@@ -129,8 +137,8 @@ cov_tc_kernel(const __grid_constant__ CUtensorMap mapX, const CovParams p) {
                 uint8_t* st = smem + s * stage_bytes;
                 mbar_arrive_expect_tx(&full[s], stage_bytes);
                 if (dup) {
-                    tma_load_5d_cov(st, &mapX, &full[s], 0, tx * 32, ty * 2, img, 0);                  // rows 0..63   : hi
-                    tma_load_5d_cov(st + Cfg::SLICE, &mapX, &full[s], 0, tx * 32, ty * 2, img, 1);     // rows 64..127 : lo
+                    tma_load_5d_cov(st, &mapX, &full[s], 0, tx * 32, ty * 2, frame, 0);                  // rows 0..63   : hi
+                    tma_load_5d_cov(st + Cfg::SLICE, &mapX, &full[s], 0, tx * 32, ty * 2, frame, 1);     // rows 64..127 : lo
                     continue;
                 }
                 for (int op = 0; op < (diag ? 1 : 2); ++op) {
@@ -139,7 +147,7 @@ cov_tc_kernel(const __grid_constant__ CUtensorMap mapX, const CovParams p) {
                         const int ch = blk * 128 + sl * 64;
                         for (int pl = 0; pl < 2; ++pl)
                             tma_load_5d_cov(st + op * Cfg::OPER + (pl * 2 + sl) * Cfg::SLICE, &mapX, &full[s], ch, tx * 32,
-                                            ty * 2, img, pl);
+                                            ty * 2, frame, pl);
                     }
                 }
             }
@@ -260,8 +268,15 @@ cov_tc_kernel(const __grid_constant__ CUtensorMap mapX, const CovParams p) {
                         for (int k = 0; k < 2; ++k) {
                             const int r = rg + 32 * k;
                             const int x = tx * 32 + (r & 31), y = ty * 2 + (r >> 5);
-                            if (x < p.W && y < p.H) {           // out-of-range pixels were zero-filled by TMA and must stay zero
-                                const int off = r * 128 + pchunk;
+                            const int off = r * 128 + pchunk;
+                            if (REG && x < p.W && y < p.H && p.labels[((long long)frame * p.H + y) * p.W + x] != region) {
+                                // another region's pixel: zero, so that it adds nothing to S or s
+                                Half8 z;
+#pragma unroll
+                                for (int j = 0; j < 4; ++j) z.v[j] = __float2half2_rn(0.f);
+                                *reinterpret_cast<Half8*>(hi_base + off) = z;
+                                *reinterpret_cast<Half8*>(lo_base + off) = z;
+                            } else if (x < p.W && y < p.H) {    // out-of-range pixels were zero-filled by TMA and must stay zero
                                 const Half8 h = *reinterpret_cast<const Half8*>(hi_base + off);
                                 const Half8 l = *reinterpret_cast<const Half8*>(lo_base + off);
                                 float v[8];
@@ -337,15 +352,66 @@ cov_tc_kernel(const __grid_constant__ CUtensorMap mapX, const CovParams p) {
     if (warp == 1) tmem_dealloc(tmem_base, 512);
 }
 
+// Region form of k_sample_shift: item n = frame * R + region; the mean of the sampled pixels OF THE REGION.  A region the
+// sample misses (a few pixels) takes the mean of all its pixels (stride 1); an empty region gets t = 0.
+__device__ __noinline__ void k_sample_shift_region(const __half* __restrict__ act, const ActGeom& g, int stride,
+                                                   float* __restrict__ shift, const uint8_t* __restrict__ labels, int R,
+                                                   float (*red)[64]) {
+    __shared__ int cnt_red[32];
+    const int grp = threadIdx.x & 7, rl = threadIdx.x >> 3;
+    const int c0 = blockIdx.x * 64 + grp * 8;
+    const int item = blockIdx.y, frame = item / R, region = item - frame * R;
+    const long long HW = (long long)g.H * g.W;
+    const uint8_t* lab = labels + (long long)frame * HW;
+    float s[8];
+    int cnt = 0;
+    for (int pass = 0; pass < 2; ++pass) {
+        const int str = pass == 0 ? stride : 1;
+        const long long ns = (HW + str - 1) / str;
+#pragma unroll
+        for (int j = 0; j < 8; ++j) s[j] = 0.f;
+        int c = 0;
+        for (long long k = rl; k < ns; k += 32) {
+            const long long q = k * str;
+            if (lab[q] != region) continue;
+            const int y = (int)(q / g.W), x = (int)(q - (long long)y * g.W);
+            float v[8];
+            load8(act, g, ((long long)frame * g.Hp + y + 1) * g.Wp + x + 1, c0, v);
+#pragma unroll
+            for (int j = 0; j < 8; ++j) s[j] += v[j];
+            ++c;
+        }
+#pragma unroll
+        for (int j = 0; j < 8; ++j) red[rl][grp * 8 + j] = s[j];
+        if (grp == 0) cnt_red[rl] = c;
+        __syncthreads();
+        cnt = 0;
+        for (int r = 0; r < 32; ++r) cnt += cnt_red[r];
+        if (cnt > 0 || str == 1) break;
+        __syncthreads();
+    }
+    if (threadIdx.x < 64) {
+        float a = 0.f;
+#pragma unroll
+        for (int r = 0; r < 32; ++r) a += red[r][threadIdx.x];
+        shift[(long long)item * g.C + blockIdx.x * 64 + threadIdx.x] = cnt > 0 ? a / (float)cnt : 0.f;
+    }
+}
+
 // shift[n][c] = mean of <= ~1024 strided interior pixels (all pixels when HW <= 1024): fixed-order reduction.
 // grid (C/64, N): one CTA per 64 channels of an image (a single CTA per image took 180 us at C = 512);
 // 256 threads = 8 channel groups x 32 pixel lanes
 __global__ void __launch_bounds__(256)
-k_sample_shift(const __half* __restrict__ act, ActGeom g, int stride, float* __restrict__ shift) {
+k_sample_shift(const __half* __restrict__ act, ActGeom g, int stride, float* __restrict__ shift, const uint8_t* __restrict__ labels,
+               int R) {
     __shared__ float red[32][64];
     const int grp = threadIdx.x & 7, rl = threadIdx.x >> 3;
     const int c0 = blockIdx.x * 64 + grp * 8;
     const int n = blockIdx.y;
+    if (labels) {
+        k_sample_shift_region(act, g, stride, shift, labels, R, red);
+        return;
+    }
     const long long HW = (long long)g.H * g.W;
     const long long ns = (HW + stride - 1) / stride;
     float s[8];
@@ -373,24 +439,31 @@ k_sample_shift(const __half* __restrict__ act, ActGeom g, int stride, float* __r
 
 // dsum[n][c] = sum over splits of psum (fp64, fixed order); mean = shift + dsum / HW
 __global__ void k_cov_sums(const float* __restrict__ psum, const float* __restrict__ shift, int C, int ksplit, long long HW,
-                           int total, double* __restrict__ dsum, float* __restrict__ mean) {
+                           int total, double* __restrict__ dsum, float* __restrict__ mean, const int* __restrict__ counts) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= total) return;
     const int n = i / C, c = i - n * C;
     double a = 0.0;
     for (int s = 0; s < ksplit; ++s) a += (double)psum[((long long)n * ksplit + s) * C + c];
     dsum[i] = a;
-    mean[i] = (float)((double)shift[i] + a / (double)HW);
+    const long long cnt = counts ? (long long)counts[n] : HW;      // regions: the pixels of the item's region
+    mean[i] = cnt > 0 ? (float)((double)shift[i] + a / (double)cnt) : shift[i];
 }
 
 // G = (sum_slots part - s s^T / HW) / (HW - 1) + eps_cov * I   (ops.py:45,50,108,121), exactly symmetric
-__global__ void k_cov_finalize(const float* __restrict__ part, const double* __restrict__ dsum, int C, int nslots, long long HW,
-                               float eps_cov, int count, float* __restrict__ G, float* __restrict__ A0) {
+__global__ void k_cov_finalize(const float* __restrict__ part, const double* __restrict__ dsum, int C, int nslots, long long HW0,
+                               float eps_cov, int count, float* __restrict__ G, float* __restrict__ A0, const int* __restrict__ counts) {
     const long long total = (long long)count * C * C;
     for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (long long)gridDim.x * blockDim.x) {
         const int j = (int)(t % C);
         const int i = (int)((t / C) % C);
         const long long n = t / ((long long)C * C);
+        const long long HW = counts ? (long long)counts[n] : HW0;
+        if (HW < 2) {                 // a region of < 2 pixels: 1/(n-1) is undefined; its pixels are copied, never transformed
+            G[t] = 0.f;
+            if (A0) A0[t] = 0.f;
+            continue;
+        }
         // every (min,max) entry lies in a stored upper block: reading it for both (i,j) and (j,i) makes G exactly symmetric
         const long long e = (i <= j) ? (long long)i * C + j : (long long)j * C + i;
         const float* pp = part + n * nslots * (long long)C * C + e;
@@ -423,7 +496,10 @@ int g_cov_max_stages = 12;   // probe knob (wctb200_debug_set_cov_stages)
 
 // Means and covariance (+ eps_cov I) of a feature batch: mean [N][C], G [N][C][C] (and a copy A0 if not null), fp32.
 // dsum: [N][C] fp64 scratch (caller's workspace); partial products live in the per-stream scratch cache.
-int launch_mean_cov(const __half* act, ActGeom g, float eps_cov, float* mean, float* G, float* A0, double* dsum, cudaStream_t st) {
+// labels / R / counts (optional): statistics per (frame, region) item, n = frame * R + region, over the pixels whose label
+// [frame][y][x] is the region; counts [N*R] = those pixel counts (k_region_counts); outputs are [N*R][...].
+int launch_mean_cov(const __half* act, ActGeom g, float eps_cov, float* mean, float* G, float* A0, double* dsum, cudaStream_t st,
+                    const uint8_t* labels, int R, const int* counts) {
     static PFN_encodeTiledC enc = nullptr;
     if (!enc) {
         void* ptr = nullptr;
@@ -437,8 +513,12 @@ int launch_mean_cov(const __half* act, ActGeom g, float eps_cov, float* mean, fl
     }
     WCTB_REQUIRE(g.C == 64 || (g.C % 128 == 0 && g.C <= 2048), "covariance: C=%d must be 64 or a multiple of 128 (<= 2048)", g.C);
     const long long HW = (long long)g.H * g.W;
+    if (!labels) R = 1;
+    const int items = g.N * R;
     CovParams p;
     p.C = g.C; p.W = g.W; p.H = g.H; p.N = g.N;
+    p.labels = labels;
+    p.R = R;
     p.tiles_x = (g.W + 31) / 32;
     p.tiles_y = (g.H + 1) / 2;
     p.nb = g.C == 64 ? 1 : g.C / 128;
@@ -454,8 +534,8 @@ int launch_mean_cov(const __half* act, ActGeom g, float eps_cov, float* mean, fl
     p.ksplit = (tiles_img + tps - 1) / tps;
     p.nslots = g.C == 64 ? 4 * p.ksplit : p.ksplit;
     // scratch: shift [N][C] | psum [N][ksplit][C] | part [N][nslots][C][C]
-    const size_t n_shift = (size_t)g.N * g.C, n_psum = (size_t)g.N * p.ksplit * g.C;
-    const size_t n_part = (size_t)g.N * p.nslots * g.C * g.C;
+    const size_t n_shift = (size_t)items * g.C, n_psum = (size_t)items * p.ksplit * g.C;
+    const size_t n_part = (size_t)items * p.nslots * g.C * g.C;
     float* scratch = nullptr;
     { int rc0 = scratch_alloc(reinterpret_cast<void**>(&scratch), (n_shift + n_psum + n_part + 64) * sizeof(float), st, 0); if (rc0) return rc0; }
     float* shift = scratch;
@@ -467,7 +547,7 @@ int launch_mean_cov(const __half* act, ActGeom g, float eps_cov, float* mean, fl
     // (blocks below the diagonal are never written -- and never read: k_cov_finalize only touches (min,max) entries)
 
     const int stride = HW <= 1024 ? 1 : (int)(HW / 1024);
-    k_sample_shift<<<dim3((unsigned)(g.C / 64), (unsigned)g.N), 256, 0, st>>>(act, g, stride, shift);
+    k_sample_shift<<<dim3((unsigned)(g.C / 64), (unsigned)items), 256, 0, st>>>(act, g, stride, shift, labels, R);
     WCTB_CHECK_LAUNCH("k_sample_shift");
 
     // tensor map over the interior pixels only (see header comment)
@@ -485,15 +565,22 @@ int launch_mean_cov(const __half* act, ActGeom g, float eps_cov, float* mean, fl
         set_error("cov_tc: cuTensorMapEncodeTiled failed (%d)", (int)r);
         return WCTB200_ECUDA;
     }
-    WCTB_ENSURE_SMEM(cov_tc_kernel, CovCfg::SMEM_BYTES);
-    dim3 grid((unsigned)(npairs * p.ksplit), (unsigned)g.N);
-    cov_tc_kernel<<<grid, CovCfg::THREADS, CovCfg::SMEM_BYTES, st>>>(mX, p);
+    dim3 grid((unsigned)(npairs * p.ksplit), (unsigned)items);
+    if (labels) {
+        WCTB_ENSURE_SMEM(cov_tc_kernel<true>, CovCfg::SMEM_BYTES);
+        cov_tc_kernel<true><<<grid, CovCfg::THREADS, CovCfg::SMEM_BYTES, st>>>(mX, p);
+    } else {
+        WCTB_ENSURE_SMEM(cov_tc_kernel<false>, CovCfg::SMEM_BYTES);
+        cov_tc_kernel<false><<<grid, CovCfg::THREADS, CovCfg::SMEM_BYTES, st>>>(mX, p);
+    }
     WCTB_CHECK_LAUNCH("cov_tc_kernel");
-    k_cov_sums<<<cdiv((long long)g.N * g.C, 256), 256, 0, st>>>(psum, shift, g.C, p.ksplit, HW, g.N * g.C, dsum, mean);
+    k_cov_sums<<<cdiv((long long)items * g.C, 256), 256, 0, st>>>(psum, shift, g.C, p.ksplit, HW, items * g.C, dsum, mean,
+                                                                   labels ? counts : nullptr);
     WCTB_CHECK_LAUNCH("k_cov_sums");
-    const long long tot = (long long)g.N * g.C * g.C;
+    const long long tot = (long long)items * g.C * g.C;
     k_cov_finalize<<<(unsigned)(cdiv(tot, 256) > 4096 ? 4096 : cdiv(tot, 256)), 256, 0, st>>>(part, dsum, g.C, p.nslots, HW,
-                                                                                               eps_cov, g.N, G, A0);
+                                                                                               eps_cov, items, G, A0,
+                                                                                               labels ? counts : nullptr);
     WCTB_CHECK_LAUNCH("k_cov_finalize");
     return 0;
 }

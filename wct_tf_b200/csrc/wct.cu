@@ -22,7 +22,9 @@ namespace wctb {
 // ---------------------------------------------------------------------------
 template <bool SQ>
 __global__ void __launch_bounds__(256)
-k_chan_sums(const __half* __restrict__ act, ActGeom g, int chunk_pix, double* __restrict__ sum, double* __restrict__ sumsq) {
+k_chan_sums(const __half* __restrict__ act, ActGeom g, int chunk_pix, double* __restrict__ sum, double* __restrict__ sumsq,
+            const uint8_t* __restrict__ labels = nullptr) {
+    // labels (optional, [N][H][W]): grid.z = R regions, sums of the pixels labelled blockIdx.z into item n * R + region
     __shared__ float red[256 * 8];
     __shared__ float red2[SQ ? 256 * 8 : 8];
     const int cgs = g.C / 8;
@@ -30,6 +32,8 @@ k_chan_sums(const __half* __restrict__ act, ActGeom g, int chunk_pix, double* __
     const int grp = threadIdx.x % cgs;
     const int rl = threadIdx.x / cgs;
     const int n = blockIdx.y;
+    const int region = blockIdx.z;
+    const long long item = (long long)n * gridDim.z + region;
     const long long HW = (long long)g.H * g.W;
     const long long q0 = (long long)blockIdx.x * chunk_pix;
     const long long q1 = min(q0 + chunk_pix, HW);
@@ -38,6 +42,7 @@ k_chan_sums(const __half* __restrict__ act, ActGeom g, int chunk_pix, double* __
     for (int j = 0; j < 8; ++j) { s[j] = 0.f; s2[j] = 0.f; }
     if (rl < rows) {
         for (long long q = q0 + rl; q < q1; q += rows) {
+            if (labels && labels[(long long)n * HW + q] != region) continue;
             const int y = (int)((unsigned)q / (unsigned)g.W), x = (int)((unsigned)q - (unsigned)y * (unsigned)g.W);
             float v[8];
             load8(act, g, ((long long)n * g.Hp + y + 1) * g.Wp + x + 1, grp * 8, v);
@@ -62,15 +67,17 @@ k_chan_sums(const __half* __restrict__ act, ActGeom g, int chunk_pix, double* __
             a += red[(r * cgs + gq) * 8 + j];
             if (SQ) a2 += red2[(r * cgs + gq) * 8 + j];
         }
-        atomicAdd(&sum[(long long)n * g.C + c], (double)a);
-        if (SQ) atomicAdd(&sumsq[(long long)n * g.C + c], (double)a2);
+        atomicAdd(&sum[item * g.C + c], (double)a);
+        if (SQ) atomicAdd(&sumsq[item * g.C + c], (double)a2);
     }
 }
 
-__global__ void k_mean_finalize(const double* __restrict__ sum, const double* __restrict__ sumsq, long long HW, int total,
-                                float* __restrict__ mean, float* __restrict__ var) {
+__global__ void k_mean_finalize(const double* __restrict__ sum, const double* __restrict__ sumsq, long long HW0, int total,
+                                float* __restrict__ mean, float* __restrict__ var, const int* __restrict__ counts = nullptr,
+                                int C = 1) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= total) return;
+    const long long HW = counts ? (counts[i / C] > 0 ? counts[i / C] : 1) : HW0;   // regions: pixels of item i / C
     const double m = sum[i] / (double)HW;
     mean[i] = (float)m;
     if (var) var[i] = (float)fmax(sumsq[i] / (double)HW - m * m, 0.0);   // biased variance (tf.nn.moments)
@@ -535,7 +542,7 @@ __global__ void k_finalize_transform(const float* __restrict__ T, int C, int Nc,
     if (row >= C) return;
     const float* t = T + ((long long)z * C + row) * C;
     const float* mc = mean_c + (long long)z * C;
-    const float* ms = mean_s + (long long)(Ns == 1 ? 0 : z) * C;
+    const float* ms = mean_s + (long long)(z % Ns) * C;          // Ns = 1 (shared), Nc (per frame) or R (item z = frame*R + region)
     __half* mh = Msplit + (((long long)z * 2 + 0) * C + row) * C;
     __half* ml = Msplit + (((long long)z * 2 + 1) * C + row) * C;
     float dot = 0.f;
@@ -561,7 +568,7 @@ __global__ void k_adain_coeffs(const float* __restrict__ mean_c, const float* __
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= Nc * C) return;
     const int z = i / C, c = i % C;
-    const int si = (Ns == 1 ? 0 : z) * C + c;
+    const int si = (z % Ns) * C + c;                                // Ns = 1, Nc, or R (item z = frame*R + region)
     const float inv = rsqrtf(var_c[i] + eps) * sqrtf(var_s[si]);   // batch_normalization(scale=sqrt(style_var))
     // y = (x - mc)*inv + ms ; out = alpha*y + (1-alpha)*x
     scale[i] = alpha * inv + (1.f - alpha);
@@ -706,7 +713,8 @@ int launch_eig_post(const float* G, const float* A0, float* lam, int C, int coun
 int launch_matfun_ns(const float* A, int C, int count, int n_first, float thresh, float eps_eig, float* out, int* ok, int* kcount,
                      cudaStream_t st, float* info = nullptr);
 // cov_tc.cu: per-channel means and covariance (+ eps_cov I) in one pass over the features
-int launch_mean_cov(const __half* act, ActGeom g, float eps_cov, float* mean, float* G, float* A0, double* dsum, cudaStream_t st);
+int launch_mean_cov(const __half* act, ActGeom g, float eps_cov, float* mean, float* G, float* A0, double* dsum, cudaStream_t st,
+                    const uint8_t* labels = nullptr, int R = 1, const int* counts = nullptr);
 
 int launch_wct_level(const __half* content, int Nc, int Hc, int Wc, const __half* style, int Ns, int Hs, int Ws, int C,
                      float alpha, float eps_cov, float eps_eig, float thresh, int readd, __half* out, int32_t* k_out,
@@ -1197,6 +1205,306 @@ int launch_style_swap_level(const __half* content, int Hc, int Wc, const __half*
     k_blend2<<<swap_grid((long long)Hc * Wc * (C / 8), 256), 256, 0, st>>>(tmp, content, gc, alpha, 1.f - alpha, out);   // ops.py:210
     WCTB_CHECK_LAUNCH("k_blend2");
     if (k_out) WCTB_CUDA(cudaMemcpyAsync(k_out, kc, 2 * 4, cudaMemcpyDeviceToDevice, st));
+    return 0;
+}
+
+// ---------------------------------------------------------------------------
+// Spatial control (Li et al. 2017, sec. 4): a uint8 label map splits every frame into regions; region r < R is whitened
+// with its OWN statistics and coloured with style r, labels >= R ("keep") and regions of < 2 pixels leave the level equal
+// by value to its input.  Item i = frame * R + region runs through the unchanged content chain of launch_wct_apply
+// (means / covariance over the region's pixels, A^-1/2, W_c, T = C_s[r] W_c[i], M, bias); the tcgen05 apply multiplies
+// (tile, region) pairs and stores only the region's pixels; k_copy_keep writes the rest.
+// ---------------------------------------------------------------------------
+
+// nearest-neighbour label resize in exact integer arithmetic: dst[n][y][x] = src[n][(y*Hs) div Hd][(x*Ws) div Wd]
+__global__ void k_labels_nearest(const uint8_t* __restrict__ src, int N, int Hs, int Ws, int Hd, int Wd, uint8_t* __restrict__ dst) {
+    const long long total = (long long)N * Hd * Wd;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+        const int x = (int)(i % Wd);
+        const long long r = i / Wd;
+        const int y = (int)(r % Hd);
+        const long long n = r / Hd;
+        const int sy = (int)(((long long)y * Hs) / Hd), sx = (int)(((long long)x * Ws) / Wd);
+        dst[i] = src[(n * Hs + sy) * Ws + sx];
+    }
+}
+int launch_labels_nearest(const uint8_t* src, int N, int Hs, int Ws, int Hd, int Wd, uint8_t* dst, cudaStream_t st) {
+    const long long total = (long long)N * Hd * Wd;
+    long long blocks = (total + 255) / 256;
+    if (blocks > device_sm_count() * 16ll) blocks = device_sm_count() * 16ll;
+    k_labels_nearest<<<(unsigned)blocks, 256, 0, st>>>(src, N, Hs, Ws, Hd, Wd, dst);
+    WCTB_CHECK_LAUNCH("k_labels_nearest");
+    return 0;
+}
+
+// counts[n*R + r] = pixels of frame n labelled r (integer sums in a fixed order: deterministic).  grid N, 256 threads.
+__global__ void __launch_bounds__(256) k_region_counts(const uint8_t* __restrict__ labels, long long HW, int R, int* __restrict__ counts) {
+    __shared__ int red[8][256];
+    const int n = blockIdx.x;
+    int c[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    const uint8_t* lab = labels + (long long)n * HW;
+    for (long long q = threadIdx.x; q < HW; q += 256) {
+        const int l = lab[q];
+#pragma unroll
+        for (int r = 0; r < 8; ++r) c[r] += (l == r) ? 1 : 0;
+    }
+#pragma unroll
+    for (int r = 0; r < 8; ++r) red[r][threadIdx.x] = c[r];
+    __syncthreads();
+    if (threadIdx.x < R) {
+        int a = 0;
+        for (int t = 0; t < 256; ++t) a += red[threadIdx.x][t];
+        counts[n * R + threadIdx.x] = a;
+    }
+}
+
+// tilemask[n][t] bit r: the 128 padded positions [t*128, t*128+128) of frame n's plane hold an interior pixel of region r
+// with >= 2 pixels (those are transformed by the apply; everything else is copied).  One warp per tile.
+__global__ void k_tile_mask(const uint8_t* __restrict__ labels, ActGeom g, int R, const int* __restrict__ counts, int tiles_per_image,
+                            uint32_t* __restrict__ tilemask) {
+    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+    if (warp >= g.N * tiles_per_image) return;
+    const int n = warp / tiles_per_image, t = warp - n * tiles_per_image;
+    const int HpWp = g.Hp * g.Wp;
+    uint32_t bits = 0u;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        const int pos = t * 128 + k * 32 + lane;
+        if (pos >= HpWp) continue;
+        const int yy = pos / g.Wp, xx = pos - yy * g.Wp;
+        if (yy < 1 || yy > g.H || xx < 1 || xx > g.W) continue;
+        const int l = labels[((long long)n * g.H + yy - 1) * g.W + xx - 1];
+        if (l < R && counts[n * R + l] >= 2) bits |= 1u << l;
+    }
+    bits = __reduce_or_sync(0xffffffffu, bits);
+    if (lane == 0) tilemask[warp] = bits;
+}
+
+// pixels the transform leaves alone (label >= R, or a region of < 2 pixels): copy both fp16 planes (+ the halo cells that
+// mirror them) -- equal by value to the input
+__global__ void k_copy_keep(const __half* __restrict__ in, ActGeom g, const uint8_t* __restrict__ labels, int R,
+                            const int* __restrict__ counts, __half* __restrict__ out) {
+    const int cgs = g.C / 8;
+    const long long total = (long long)g.N * g.H * g.W * cgs;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+        const long long pix = i / cgs;
+        const int c0 = (int)(i - pix * cgs) * 8;
+        const int l = labels[pix];
+        const int x = (int)(pix % g.W);
+        const long long r = pix / g.W;
+        const int y = (int)(r % g.H);
+        const int n = (int)(r / g.H);
+        if (l < R && counts[n * R + l] >= 2) continue;
+        const long long off = (((long long)n * g.Hp + y + 1) * g.Wp + x + 1) * g.C + c0;
+        const Half8 hi = *reinterpret_cast<const Half8*>(in + off);
+        const Half8 lo = *reinterpret_cast<const Half8*>(in + g.plane + off);
+        store8_with_halo(out, g, n, y, x, c0, hi, lo);
+    }
+}
+
+// AdaIN per region: item n*R + label's affine map; keep pixels copied
+__global__ void k_affine_apply_regions(const __half* __restrict__ in, ActGeom g, const uint8_t* __restrict__ labels, int R,
+                                       const int* __restrict__ counts, const float* __restrict__ scale, const float* __restrict__ shift,
+                                       __half* __restrict__ out) {
+    const int cgs = g.C / 8;
+    const long long total = (long long)g.N * g.H * g.W * cgs;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+        const long long pix = i / cgs;
+        const int c0 = (int)(i - pix * cgs) * 8;
+        const int l = labels[pix];
+        const int x = (int)(pix % g.W);
+        const long long r = pix / g.W;
+        const int y = (int)(r % g.H);
+        const int n = (int)(r / g.H);
+        const long long off = (((long long)n * g.Hp + y + 1) * g.Wp + x + 1) * g.C + c0;
+        Half8 hi = *reinterpret_cast<const Half8*>(in + off);
+        Half8 lo = *reinterpret_cast<const Half8*>(in + g.plane + off);
+        if (l < R && counts[n * R + l] >= 2) {
+            float v[8];
+            merge8(hi, lo, v);
+            const float* sc = scale + ((long long)n * R + l) * g.C + c0;
+            const float* sh = shift + ((long long)n * R + l) * g.C + c0;
+#pragma unroll
+            for (int j = 0; j < 8; ++j) v[j] = fmaf(v[j], sc[j], sh[j]);
+            split8(v, hi, lo);
+        }
+        store8_with_halo(out, g, n, y, x, c0, hi, lo);
+    }
+}
+
+// workspace: the content chain of Nc*R items (wct_layout(C, Nc*R, 0)) | style means [R][C] | pixel counts [Nc*R] |
+// AdaIN style sums [2][R][C] fp64 and style mean / variance [2][R][C]
+struct RegionWs {
+    WctWs base;
+    size_t ms, counts, ssum, smv, total;
+};
+static RegionWs regions_layout(int C, int Nc, int R) {
+    RegionWs L;
+    L.base = wct_layout(C, Nc * R, 0);
+    size_t o = L.base.total;
+    auto take = [&](size_t bytes) { size_t r = o; o = align_up(o + bytes, 256); return r; };
+    L.ms = take((size_t)R * C * 4);
+    L.counts = take((size_t)Nc * R * 4);
+    L.ssum = take((size_t)2 * R * C * 8);
+    L.smv = take((size_t)2 * R * C * 4);
+    L.total = o;
+    return L;
+}
+size_t wct_regions_workspace_bytes(int C, int Nc, int R) { return regions_layout(C, Nc, R).total; }
+
+static int launch_region_counts(const uint8_t* labels, int Nc, int Hc, int Wc, int R, int* counts, cudaStream_t st) {
+    k_region_counts<<<(unsigned)Nc, 256, 0, st>>>(labels, (long long)Hc * Wc, R, counts);
+    WCTB_CHECK_LAUNCH("k_region_counts");
+    return 0;
+}
+
+static int launch_copy_keep(const __half* content, ActGeom gc, const uint8_t* labels, int R, const int* counts, __half* out,
+                            cudaStream_t st) {
+    const long long total = (long long)gc.N * gc.H * gc.W * (gc.C / 8);
+    long long blocks = (total + 255) / 256;
+    if (blocks > device_sm_count() * 16ll) blocks = device_sm_count() * 16ll;
+    k_copy_keep<<<(unsigned)blocks, 256, 0, st>>>(content, gc, labels, R, counts, out);
+    WCTB_CHECK_LAUNCH("k_copy_keep");
+    return 0;
+}
+
+int launch_wct_apply_regions(const __half* content, int Nc, int Hc, int Wc, int C, const uint8_t* labels, int R,
+                             const void* const* states, float alpha, float eps_cov, float eps_eig, float thresh, int readd,
+                             __half* out, int32_t* k_out, void* ws, size_t ws_bytes, cudaStream_t st) {
+    WCTB_REQUIRE(C == 64 || C == 128 || C == 256 || C == 512, "wct_apply_regions: C=%d not in {64,128,256,512}", C);
+    WCTB_REQUIRE(R >= 1 && R <= 8, "wct_apply_regions: R=%d not in 1..8", R);
+    for (int r = 0; r < R; ++r) WCTB_REQUIRE(states[r] != nullptr, "wct_apply_regions: style state %d is NULL", r);
+    const RegionWs RL = regions_layout(C, Nc, R);
+    if (ws_bytes < RL.total) {
+        set_error("wct_apply_regions: workspace %zu < %zu bytes", ws_bytes, RL.total);
+        return WCTB200_EWS;
+    }
+    const WctWs& L = RL.base;
+    const int NR = Nc * R;
+    uint8_t* w = static_cast<uint8_t*>(ws);
+    size_t off_cs, off_k;
+    style_state_offsets(C, 1, &off_cs, &off_k);
+    double* dsum = reinterpret_cast<double*>(w + L.dsum);
+    float* mean = reinterpret_cast<float*>(w + L.mean);
+    float* G = reinterpret_cast<float*>(w + L.G);
+    float* A0 = reinterpret_cast<float*>(w + L.A0);
+    float* lam = reinterpret_cast<float*>(w + L.lam);
+    float* sigma = reinterpret_cast<float*>(w + L.sigma);
+    float* dvec = reinterpret_cast<float*>(w + L.dvec);
+    float* Wcm = reinterpret_cast<float*>(w + L.Wc);
+    float* T = reinterpret_cast<float*>(w + L.T);
+    __half* Msplit = reinterpret_cast<__half*>(w + L.Msplit);
+    float* bias = reinterpret_cast<float*>(w + L.bias);
+    float* conv = reinterpret_cast<float*>(w + L.conv);
+    int* kc = reinterpret_cast<int*>(w + L.kcount);
+    int* ok = reinterpret_cast<int*>(w + L.ok);
+    float* ms_all = reinterpret_cast<float*>(w + RL.ms);
+    int* counts = reinterpret_cast<int*>(w + RL.counts);
+    const long long CC = (long long)C * C;
+    const ActGeom gc(Nc, Hc, Wc, C);
+    const int tpi = cdiv((long long)gc.Hp * gc.Wp, 128);
+    uint32_t* tilemask = nullptr;
+    { int rc0 = scratch_alloc(reinterpret_cast<void**>(&tilemask), (size_t)Nc * tpi * 4, st, 3); if (rc0) return rc0; }
+
+    WCTB_CUDA(cudaMemsetAsync(kc, 0, (size_t)NR * 2 * 4, st));
+    int rc = launch_region_counts(labels, Nc, Hc, Wc, R, counts, st);
+    if (rc) return rc;
+    rc = launch_mean_cov(content, gc, eps_cov, mean, G, A0, dsum, st, labels, R, counts);
+    if (rc) return rc;
+    rc = launch_matfun_ns(A0, C, NR, /*n_first=*/NR, thresh, eps_eig, Wcm, ok, kc, st);   // W_c = A^-1/2 where every eigenvalue is kept
+    if (rc < 0) return rc;
+    rc = launch_jacobi(G, C, NR, conv, kc + NR, st, ok);
+    if (rc) return rc;
+    rc = launch_eig_post(G, A0, lam, C, NR, thresh, eps_eig, NR, sigma, dvec, kc, st, ok);
+    if (rc) return rc;
+    dim3 gg((unsigned)(C / 64), (unsigned)(C / 64), (unsigned)NR);
+    k_outer_gemm<<<gg, 256, 0, st>>>(G, CC, G, CC, dvec, C, Wcm, CC, C, ok);
+    WCTB_CHECK_LAUNCH("k_outer_gemm(Wc)");
+    // T[n*R + r] = C_s[r] W_c[n*R + r]: one launch per region (strides R*C*C over the frames)
+    dim3 gt((unsigned)(C / 64), (unsigned)(C / 64), (unsigned)Nc);
+    for (int r = 0; r < R; ++r) {
+        const uint8_t* sp = static_cast<const uint8_t*>(states[r]);
+        WCTB_CUDA(cudaMemcpyAsync(ms_all + (long long)r * C, sp, (size_t)C * 4, cudaMemcpyDeviceToDevice, st));
+        k_outer_gemm<<<gt, 256, 0, st>>>(reinterpret_cast<const float*>(sp + off_cs), 0, Wcm + r * CC, R * CC, nullptr, 0,
+                                         T + r * CC, R * CC, C);
+        WCTB_CHECK_LAUNCH("k_outer_gemm(T)");
+    }
+    dim3 gf((unsigned)cdiv(C, 8), (unsigned)NR);
+    k_finalize_transform<<<gf, 256, 0, st>>>(T, C, NR, R, alpha, readd, mean, ms_all, Msplit, bias);
+    WCTB_CHECK_LAUNCH("k_finalize_transform");
+    k_tile_mask<<<(unsigned)cdiv((long long)Nc * tpi * 32, 256), 256, 0, st>>>(labels, gc, R, counts, tpi, tilemask);
+    WCTB_CHECK_LAUNCH("k_tile_mask");
+    rc = launch_conv_tc(CONV_APPLY, content, Nc, Hc, Wc, C, Msplit, NR, nullptr, bias, C, 0, out, st, 3, labels, R, tilemask);
+    if (rc) return rc;
+    rc = launch_copy_keep(content, gc, labels, R, counts, out, st);
+    if (rc) return rc;
+    if (k_out) {
+        // k_out: [k_c x Nc*R | n_r x Nc*R], frame-major
+        WCTB_CUDA(cudaMemcpyAsync(k_out, kc, (size_t)NR * 4, cudaMemcpyDeviceToDevice, st));
+        WCTB_CUDA(cudaMemcpyAsync(k_out + NR, counts, (size_t)NR * 4, cudaMemcpyDeviceToDevice, st));
+    }
+    return 0;
+}
+
+int launch_adain_regions(const __half* content, int Nc, int Hc, int Wc, int C, const uint8_t* labels, int R,
+                         const __half* const* styles, const int* style_hw, float alpha, float eps, __half* out, void* ws,
+                         size_t ws_bytes, cudaStream_t st) {
+    WCTB_REQUIRE(C % 8 == 0 && C <= 2048, "adain_regions: C=%d must be a multiple of 8 (<= 2048)", C);
+    WCTB_REQUIRE(R >= 1 && R <= 8, "adain_regions: R=%d not in 1..8", R);
+    for (int r = 0; r < R; ++r)
+        WCTB_REQUIRE(styles[r] != nullptr && style_hw[2 * r] >= 2 && style_hw[2 * r + 1] >= 2, "adain_regions: bad style %d", r);
+    const RegionWs RL = regions_layout(C, Nc, R);
+    if (ws_bytes < RL.total) {
+        set_error("adain_regions: workspace %zu < %zu bytes", ws_bytes, RL.total);
+        return WCTB200_EWS;
+    }
+    const WctWs& L = RL.base;
+    const int NR = Nc * R;
+    uint8_t* w = static_cast<uint8_t*>(ws);
+    double* sum = reinterpret_cast<double*>(w + L.sum);
+    double* sumsq = reinterpret_cast<double*>(w + L.sumsq);
+    float* mean = reinterpret_cast<float*>(w + L.mean);
+    float* var = reinterpret_cast<float*>(w + L.var);
+    float* scale = reinterpret_cast<float*>(w + L.scale);
+    float* shift = reinterpret_cast<float*>(w + L.shift);
+    int* counts = reinterpret_cast<int*>(w + RL.counts);
+    double* ssum = reinterpret_cast<double*>(w + RL.ssum);
+    float* smean = reinterpret_cast<float*>(w + RL.smv);
+    float* svar = smean + (long long)R * C;
+    WCTB_CUDA(cudaMemsetAsync(w + L.sum, 0, L.dsum - L.sum, st));
+    WCTB_CUDA(cudaMemsetAsync(ssum, 0, (size_t)2 * R * C * 8, st));
+    int rc = launch_region_counts(labels, Nc, Hc, Wc, R, counts, st);
+    if (rc) return rc;
+    const ActGeom gc(Nc, Hc, Wc, C);
+    {
+        // the chunking of launch_sums, one grid layer per region
+        const long long HW = (long long)Hc * Wc;
+        long long chunk = (HW * Nc + 591) / 592;
+        const int rows = 256 / (C / 8) > 0 ? 256 / (C / 8) : 1;
+        chunk = (chunk + rows - 1) / rows * rows;
+        if (chunk < rows) chunk = rows;
+        if (chunk > 1024) chunk = 1024;
+        dim3 grid((unsigned)cdiv(HW, chunk), (unsigned)Nc, (unsigned)R);
+        k_chan_sums<true><<<grid, 256, 0, st>>>(content, gc, (int)chunk, sum, sumsq, labels);
+        WCTB_CHECK_LAUNCH("k_chan_sums(regions)");
+    }
+    for (int r = 0; r < R; ++r) {
+        const ActGeom gs(1, style_hw[2 * r], style_hw[2 * r + 1], C);
+        rc = launch_sums<true>(styles[r], gs, ssum + (long long)r * C, ssum + (long long)(R + r) * C, st);
+        if (rc) return rc;
+        k_mean_finalize<<<cdiv(C, 256), 256, 0, st>>>(ssum + (long long)r * C, ssum + (long long)(R + r) * C, (long long)gs.H * gs.W,
+                                                       C, smean + (long long)r * C, svar + (long long)r * C);
+        WCTB_CHECK_LAUNCH("k_mean_finalize(s)");
+    }
+    k_mean_finalize<<<cdiv((long long)NR * C, 256), 256, 0, st>>>(sum, sumsq, 1, NR * C, mean, var, counts, C);
+    WCTB_CHECK_LAUNCH("k_mean_finalize(c)");
+    k_adain_coeffs<<<cdiv((long long)NR * C, 256), 256, 0, st>>>(mean, var, smean, svar, C, NR, R, alpha, eps, scale, shift);
+    WCTB_CHECK_LAUNCH("k_adain_coeffs");
+    const long long total = (long long)Nc * Hc * Wc * (C / 8);
+    long long blocks = (total + 255) / 256;
+    if (blocks > device_sm_count() * 16) blocks = device_sm_count() * 16;
+    k_affine_apply_regions<<<(unsigned)blocks, 256, 0, st>>>(content, gc, labels, R, counts, scale, shift, out);
+    WCTB_CHECK_LAUNCH("k_affine_apply_regions");
     return 0;
 }
 

@@ -152,6 +152,15 @@ def preserve_colors_np(style_rgb, content_rgb):
     return out
 
 
+def labels_resize(labels, H, W):
+    """Nearest-neighbour resize of cuda uint8 label maps [N,Hs,Ws] -> [N,H,W]: L[(y*Hs) div H][(x*Ws) div W]."""
+    labels = labels.contiguous()
+    N, Hs, Ws = labels.shape
+    out = torch.empty((N, H, W), dtype=torch.uint8, device=labels.device)
+    _capi.check(_capi.load().wctb200_labels_resize_nearest(labels.data_ptr(), N, Hs, Ws, H, W, out.data_ptr(), _stream()))
+    return out
+
+
 def concat_with_style(style_img, result):
     """--concat (stylize.py:107-111): [style resized to the result's height, square | result]"""
     edge = result.shape[0]

@@ -6,6 +6,8 @@ hand-written sm_100a kernel behind the C-ABI (include/wctb200.h).
 """
 from __future__ import annotations
 
+import ctypes
+
 import numpy as np
 import torch
 
@@ -318,9 +320,78 @@ class Engine(object):
                    flops=2.0 * C * C * 2 * content.N * hwc, bytes_=4.0 * C * 2 * content.N * hwc)
         return out, kbuf
 
+    # ------------------------------------------------------------------ spatial control
+    MAX_REGIONS = 8
+
+    def labels_resize(self, labels, H, W):
+        """Nearest-neighbour resize of cuda uint8 label maps [N,Hs,Ws] -> [N,H,W] (exact integer rule, include/wctb200.h)."""
+        labels = labels.contiguous()
+        N, Hs, Ws = labels.shape
+        if (Hs, Ws) == (H, W):
+            return labels
+        out = torch.empty((N, H, W), dtype=torch.uint8, device=self.device)
+        self._call("labels_nearest", 1, self.lib.wctb200_labels_resize_nearest, labels.data_ptr(), N, Hs, Ws, H, W, out.data_ptr(),
+                   self._stream())
+        return out
+
+    def _regions_workspace(self, C, Nc, R):
+        key = ("regions", self._group, C, Nc, R)
+        ws = self._ws.get(key)
+        if ws is None:
+            ws = torch.empty(self.lib.wctb200_wct_regions_workspace_bytes(C, Nc, R), dtype=torch.uint8, device=self.device)
+            self._ws[key] = ws
+        return ws
+
+    def wct_apply_regions(self, content, labels, states, alpha, want_info=False):
+        """One level with one style state per region; ``labels`` cuda uint8 [N, content.H, content.W]."""
+        st = self._stream()
+        sem = SEMANTICS[self.semantics]
+        C, R, N = content.C, len(states), content.N
+        out = self._act(N, content.H, content.W, C)
+        ws = self._regions_workspace(C, N, R)
+        kbuf = torch.empty(2 * N * R, dtype=torch.int32, device=self.device) if want_info else None
+        ptrs = (ctypes.c_void_p * R)(*[s.data_ptr() for s in states])
+        hwc = content.H * content.W
+        self._call("wct_regions[C%d]" % C, 13 + R + self._matfun_launches(C), self.lib.wctb200_wct_apply_regions, content.ptr, N,
+                   content.H, content.W, C, labels.data_ptr(), R, ctypes.cast(ptrs, ctypes.c_void_p), float(alpha), sem["eps_cov"],
+                   sem["eps_eig"], sem["thresh"], sem["readd"], out.ptr, kbuf.data_ptr() if want_info else None, ws.data_ptr(),
+                   ws.numel(), st, flops=2.0 * C * C * (R + 1) * N * hwc, bytes_=4.0 * C * (R + 1) * N * hwc)
+        return out, kbuf
+
+    def adain_regions(self, content, labels, styles, alpha):
+        st = self._stream()
+        C, R, N = content.C, len(styles), content.N
+        out = self._act(N, content.H, content.W, C)
+        ws = self._regions_workspace(C, N, R)
+        ptrs = (ctypes.c_void_p * R)(*[s.ptr for s in styles])
+        hw = (ctypes.c_int * (2 * R))(*[v for s in styles for v in (s.H, s.W)])
+        self._call("adain_regions[C%d]" % C, 6 + 2 * R, self.lib.wctb200_adain_regions, content.ptr, N, content.H, content.W, C,
+                   labels.data_ptr(), R, ctypes.cast(ptrs, ctypes.c_void_p), ctypes.cast(hw, ctypes.c_void_p), float(alpha), 1e-5,
+                   out.ptr, ws.data_ptr(), ws.numel(), st)
+        return out, None
+
+    def _check_labels(self, content_u8, styles, labels, swap5):
+        if swap5:
+            raise ValueError("style swap (swap5) cannot be combined with a label mask: it is not a per-region statistic")
+        R = len(styles)
+        if not 1 <= R <= self.MAX_REGIONS:
+            raise ValueError("a label mask takes 1..%d styles, got %d" % (self.MAX_REGIONS, R))
+        for s in styles:
+            if s.dim() != 4 or s.shape[0] != 1 or s.dtype != torch.uint8:
+                raise ValueError("each region style must be a uint8 [1,Hs,Ws,3] tensor")
+        N, H, W = content_u8.shape[:3]
+        if labels.dtype != torch.uint8 or labels.dim() != 3 or labels.shape[0] not in (1, N) or tuple(labels.shape[1:]) != (H, W):
+            raise ValueError("labels must be uint8 [N|1, %d, %d] (the content's size), got %s %s"
+                             % (H, W, tuple(labels.shape), labels.dtype))
+        if labels.device != self.device:
+            labels = labels.to(self.device)
+        if labels.shape[0] != N:
+            labels = labels.expand(N, H, W)
+        return labels.contiguous()
+
     # ------------------------------------------------------------------ pipeline
     def stylize(self, content_u8, style_u8, alpha=1.0, adain=False, want_info=False, capture=None, swap5=False, ss_alpha=0.6,
-                ss_patch_size=3, ss_stride=1):
+                ss_patch_size=3, ss_stride=1, labels=None):
         """content_u8: cuda uint8 [N,H,W,3]; style_u8: cuda uint8 [Ns,Hs,Ws,3], Ns in {1, N}.
         Returns the float32 ``decoded_output`` [N,H',W',3] (unclipped, model.py:94).
         ``capture`` (dict) receives every level's input image / features for parity tests.
@@ -328,7 +399,14 @@ class Engine(object):
         With ``self.groups`` = G > 1 the batch is cut into G sub-batches whose level chains are
         enqueued on G independent stream pairs: frames are independent (wct.py:97-103), and the
         eigendecompositions are latency bound on a few SMs, so one group's Jacobi clusters overlap the
-        other groups' convolutions (same arithmetic per frame; only the schedule changes)."""
+        other groups' convolutions (same arithmetic per frame; only the schedule changes).
+
+        ``labels`` (cuda uint8 [N|1,H,W], the content's size): spatial control.  ``style_u8`` is then a sequence of R <= 8
+        uint8 [1,Hs_r,Ws_r,3] styles; label r < R takes style r, labels >= R keep the content (include/wctb200.h)."""
+        if labels is not None:
+            styles = list(style_u8)
+            labels = self._check_labels(content_u8, styles, labels, swap5)
+            return self._stylize_regions(content_u8, styles, labels, alpha, adain, want_info, capture)
         N = content_u8.shape[0]
         swap5 = bool(swap5) and "relu5_1" in [l.relu_target for l in self.model.levels]    # model.py:148: only relu5_1 swaps
         if swap5:
@@ -376,6 +454,50 @@ class Engine(object):
             return out
         return self._stylize_one(content_u8, style_u8, alpha, adain, want_info, capture)
 
+    def _stylize_regions(self, content_u8, styles, labels, alpha, adain, want_info, capture):
+        """The masked form of ``stylize``: every style's encoder pass (and, for the WCT, its per-level preparation) runs
+        once on the style stream; with groups > 1 every sub-batch waits on those events."""
+        N = content_u8.shape[0]
+        main = torch.cuda.current_stream(self.device)
+        G = min(self.groups, N) if (capture is None and not want_info) else 1
+        if G <= 1:
+            shared = [self._style_side(s, not adain, main) for s in styles]
+            out = self._stylize_one(content_u8, None, alpha, adain, want_info, capture, labels=labels, region_styles=shared)
+            for sh in shared:
+                if sh["side"] is not main:
+                    sh["side"].wait_stream(main)
+            return out
+        self._group = 1
+        try:
+            shared = [self._style_side(s, not adain, main) for s in styles]
+        finally:
+            self._group = 0
+        bounds = [(g * N) // G for g in range(G + 1)]
+        outs = []
+        for g in range(G):
+            lo, hi = bounds[g], bounds[g + 1]
+            if g not in self._group_streams:
+                prio = -1 if (self.group_priorities and g == 0) else 0
+                self._group_streams[g] = torch.cuda.Stream(device=self.device, priority=prio)
+            gs = self._group_streams[g]
+            gs.wait_stream(main)
+            self._group = g + 1
+            try:
+                with torch.cuda.stream(gs):
+                    outs.append(self._stylize_one(content_u8[lo:hi], None, alpha, adain, False, None, labels=labels[lo:hi],
+                                                  region_styles=shared))
+            finally:
+                self._group = 0
+        for g in range(G):
+            main.wait_stream(self._group_streams[g])
+        out = torch.cat(outs, dim=0)
+        for g in range(G):
+            self._group_streams[g].wait_stream(main)
+        for sh in shared:
+            if sh["side"] is not main:
+                sh["side"].wait_stream(main)
+        return out
+
     def _style_side(self, style_u8, split, main):
         """Style side of one call (model.py:70-72: ONE encoder pass emitting every target; ops.py:48-55,76 per level when
         ``split``): enqueued on this group's style stream when overlap is on.  Returns the states / events / features."""
@@ -405,25 +527,38 @@ class Engine(object):
         return dict(states=states, events=events, feats=feats, side=side)
 
     def _stylize_one(self, content_u8, style_u8, alpha, adain, want_info, capture, swap5=False, ss_alpha=0.6, shared_style=None,
-                     ss_patch=3, ss_stride=1):
+                     ss_patch=3, ss_stride=1, labels=None, region_styles=None):
         lib, st = self.lib, self._stream()
         N = content_u8.shape[0]
-        assert content_u8.dtype == torch.uint8 and style_u8.dtype == torch.uint8
-        assert style_u8.shape[0] in (1, N)
+        assert content_u8.dtype == torch.uint8
+        assert labels is not None or (style_u8.dtype == torch.uint8 and style_u8.shape[0] in (1, N))
         content = torch.empty(content_u8.shape, dtype=torch.float32, device=self.device)
         self._call("u8_to_f32", 1, lib.wctb200_image_u8_to_f32, content_u8.data_ptr(), content_u8.numel(), content.data_ptr(), st)
         main = torch.cuda.current_stream(self.device)
         split = not adain and not swap5        # WCT: style side on its own stream; AdaIN / style swap: keep it inline
-        ss = shared_style if (shared_style is not None and split) else self._style_side(style_u8, split, main)
-        side, style_states, style_events, style_feats = ss["side"], ss["states"], ss["events"], ss["feats"]
+        if labels is None:
+            ss = shared_style if (shared_style is not None and split) else self._style_side(style_u8, split, main)
+            side, style_states, style_events, style_feats = ss["side"], ss["states"], ss["events"], ss["feats"]
+            n_style = style_u8.shape[0]
+        else:
+            side = main                        # the region styles' streams are joined by _stylize_regions
         infos = []
         x = content
         nlev = len(self.model.levels)
-        n_style = style_u8.shape[0]
         for lvl in self.model.levels:
             self._tag = lvl.relu_target
             cf, _ = self.encode(x, lvl.relu_target)
-            if swap5 and lvl.relu_target == "relu5_1":     # model.py:148-152: style swap wins over AdaIN / WCT at relu5_1
+            if labels is not None:
+                relu = lvl.relu_target
+                lab = self.labels_resize(labels, cf.H, cf.W)     # always from the call's label map (the decoder may grow odd sizes)
+                if adain:
+                    f, kbuf = self.adain_regions(cf, lab, [rs["feats"][relu] for rs in region_styles], alpha)
+                else:
+                    for rs in region_styles:
+                        if rs["side"] is not main:
+                            main.wait_event(rs["events"][relu])
+                    f, kbuf = self.wct_apply_regions(cf, lab, [rs["states"][relu] for rs in region_styles], alpha, want_info)
+            elif swap5 and lvl.relu_target == "relu5_1":     # model.py:148-152: style swap wins over AdaIN / WCT at relu5_1
                 f, kbuf = self.style_swap(cf, style_feats[lvl.relu_target], ss_alpha, want_info, ss_patch, ss_stride)
             elif split:
                 if side is not main:

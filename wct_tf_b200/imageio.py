@@ -101,3 +101,12 @@ def swap_filter_fit(H, W, patch_size, stride, n_pools=4):
     hc, wc = (hp - patch_size) // stride + 1, (wp - patch_size) // stride + 1
     hd, wd = (hc - 1) * stride + patch_size, (wc - 1) * stride + patch_size
     return (hp != hd) or (wp != wd), hd * 2 ** n_pools, wd * 2 ** n_pools
+
+
+def get_mask(path):
+    """Label mask for spatial control: an 8-bit image in mode 'L' (grey value = label) or 'P' (palette index = label).
+    Returns uint8 [H, W]; any other mode is refused."""
+    img = Image.open(path)
+    if img.mode not in ("L", "P"):
+        raise ValueError("mask %s has mode %r: a label mask must be an 8-bit 'L' (grey) or 'P' (palette) image" % (path, img.mode))
+    return np.array(img, dtype=np.uint8)

@@ -8,7 +8,8 @@ sm_100a engine (engine.py -> libwctb200.so).  Differences, all explicit:
   * ``device`` accepts the reference's TF strings ('/gpu:0') and torch strings;
   * ``swap5=True`` (style-swap at relu5_1, ops.py:145-278) honours ``ss_patch_size`` / ``ss_stride``; with a stride the
     content is centre-cropped so that the patches tile its relu5_1 encoding, as wct.py:84-90 does;
-  * ``predict_batch`` is new: a batch of frames per call (frames are independent).
+  * ``predict_batch`` is new: a batch of frames per call (frames are independent);
+  * ``labels=`` (both calls) is new: spatial control, one style per region of a uint8 label mask (Li et al. 2017, sec. 4).
 """
 from __future__ import annotations
 
@@ -67,7 +68,7 @@ class WCT(object):
         return np.uint8(np.clip(image, 0, 1) * 255)
 
     def predict_batch(self, contents, styles, alpha=1, adain=False, return_float=False, out=None, swap5=False, ss_alpha=1,
-                      passes=1, return_device=False):
+                      passes=1, return_device=False, labels=None):
         """contents: uint8 [N,H,W,3]; styles: uint8 [1|N,Hs,Ws,3] (numpy or torch; host buffers --
         ideally pinned -- or device tensors).  Returns uint8 [N,H',W',3] on the host: a numpy array,
         or ``out`` (a pinned uint8 torch tensor of the right shape) filled in place.  The call is
@@ -76,9 +77,18 @@ class WCT(object):
         ``passes`` > 1 repeats the stylisation on the previous OUTPUT like stylize.py:102-104 (``--passes``), but keeps the
         intermediate frames on the device: each pass still ends in the uint8 quantisation of wct.py:66-68 and restarts from
         /255 (wct.py:60-64), so the result is bit-identical to calling predict once per pass; style swap only acts in the
-        first pass, as in stylize_video.py:117-121.  ``return_device=True`` returns the uint8 cuda tensor instead of a host copy."""
+        first pass, as in stylize_video.py:117-121.  ``return_device=True`` returns the uint8 cuda tensor instead of a host copy.
+
+        ``labels`` (uint8 [N|1,H,W] or [H,W], the contents' size; numpy or torch): spatial control.  ``styles`` is then a
+        list of R <= 8 style images; pixels labelled r < R take style r, labels >= R keep the content.  Every pass uses the
+        same labels."""
         eng = self.engine
         dev = eng.device
+        if labels is not None:
+            if swap5:
+                raise ValueError("swap5 cannot be combined with labels: style swap is not a per-region statistic")
+            if not isinstance(styles, (list, tuple)):
+                raise ValueError("with labels, styles must be a list of R style images (one per region)")
 
         def to_dev(a):
             if isinstance(a, np.ndarray):
@@ -100,18 +110,32 @@ class WCT(object):
                     contents = center_crop_to(contents, H, W)
         with torch.cuda.device(dev):
             c = to_dev(contents)
-            s = to_dev(styles)
-            if swap5:
-                # one pair per call like the reference graph (ops.py:146); frames of a batch are swapped one by one
-                outs = [eng.stylize(c[i:i + 1], s[i:i + 1] if s.shape[0] > 1 else s, alpha=alpha, adain=adain, swap5=True,
-                                    ss_alpha=ss_alpha, ss_patch_size=self.ss_patch_size, ss_stride=self.ss_stride)
-                        for i in range(c.shape[0])]
-                out_f = outs[0] if len(outs) == 1 else torch.cat(outs, dim=0)
+            if labels is not None:
+                lab = labels if isinstance(labels, torch.Tensor) else torch.from_numpy(np.array(labels, copy=True, order="C"))
+                if lab.dim() == 2:
+                    lab = lab.unsqueeze(0)
+                if lab.dtype != torch.uint8 or lab.dim() != 3 or tuple(lab.shape[1:]) != tuple(c.shape[1:3]):
+                    raise ValueError("labels must be uint8 [N|1,H,W] with the contents' H x W = %s, got %s %s"
+                                     % (tuple(c.shape[1:3]), tuple(lab.shape), lab.dtype))
+                lab = lab.to(dev, non_blocking=True).contiguous()
+                s = [to_dev(x) for x in styles]
+                out_f = eng.stylize(c, s, alpha=alpha, adain=adain, labels=lab)
             else:
-                out_f = eng.stylize(c, s, alpha=alpha, adain=adain)
+                lab = None
+                s = to_dev(styles)
+                if swap5:
+                    # one pair per call like the reference graph (ops.py:146); frames of a batch are swapped one by one
+                    outs = [eng.stylize(c[i:i + 1], s[i:i + 1] if s.shape[0] > 1 else s, alpha=alpha, adain=adain, swap5=True,
+                                        ss_alpha=ss_alpha, ss_patch_size=self.ss_patch_size, ss_stride=self.ss_stride)
+                            for i in range(c.shape[0])]
+                    out_f = outs[0] if len(outs) == 1 else torch.cat(outs, dim=0)
+                else:
+                    out_f = eng.stylize(c, s, alpha=alpha, adain=adain)
             out_dev = eng.to_u8(out_f)
             for _ in range(int(passes) - 1):
-                out_f = eng.stylize(out_dev, s, alpha=alpha, adain=adain)
+                # an odd size grows through the decoder: the labels follow (nearest, always from the caller's map)
+                lab_p = None if lab is None else eng.labels_resize(lab, out_dev.shape[1], out_dev.shape[2])
+                out_f = eng.stylize(out_dev, s, alpha=alpha, adain=adain, labels=lab_p)
                 out_dev = eng.to_u8(out_f)
             if return_device:
                 eng.check_device()            # synchronises; raises WctB200Error if a kernel recorded a pipeline time-out
@@ -131,10 +155,13 @@ class WCT(object):
             return out_u8, out_f.cpu().numpy()
         return out_u8
 
-    def predict(self, content, style, alpha=1, swap5=False, ss_alpha=1, adain=False):
-        '''Stylize a single content/style pair (wct.py:70-106).'''
+    def predict(self, content, style, alpha=1, swap5=False, ss_alpha=1, adain=False, labels=None):
+        '''Stylize a single content/style pair (wct.py:70-106); with ``labels`` ([H,W] uint8), ``style`` is a list of R
+        styles, one per region.'''
         s = time.time()
-        out = self.predict_batch(np.asarray(content), np.asarray(style), alpha=alpha, adain=adain, swap5=swap5, ss_alpha=ss_alpha)
+        styles = [np.asarray(x) for x in style] if labels is not None else np.asarray(style)
+        out = self.predict_batch(np.asarray(content), styles, alpha=alpha, adain=adain, swap5=swap5, ss_alpha=ss_alpha,
+                                 labels=None if labels is None else np.asarray(labels))
         if self.verbose:
             print("Stylized in:", time.time() - s)   # wct.py:104
         return out[0]
